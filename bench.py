@@ -7,6 +7,7 @@ workload 2-D Poisson, N = 16385 (268M DOF), V(2,2) weighted Jacobi omega = 2/3, 
 step     one complete solve (reset phi to 0, cycle until converged, residual norm every cycle).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]          our CUDA path
+  python bench.py ... --dump-outputs bench_outputs             also write the last timed solve's results there (.npy)
   python bench.py --impl reference ...                         the reference's CPU path (oracle/_ref)
 
 `value` is measured with f resident in HBM; `e2e` goes through the C ABI with pinned HOST buffers
@@ -238,6 +239,24 @@ def pinned(pmg, shape):
     return np.frombuffer(buf, dtype=np.float64).reshape(shape), p
 
 
+DUMP_SAMPLE_POINTS = 1 << 22  # 32 MB of float64: the solution is 2.1 GB at N = 16385
+
+
+def dump_outputs(out_dir, phi, hist):
+    """--dump-outputs: what the last timed solve returned, as float64 .npy files.
+      residual_history.npy   ||r|| before cycle 1 and after every cycle (its length is the cycle count + 1)
+      solution.npy           the whole N x N solution, when it has at most DUMP_SAMPLE_POINTS points; otherwise
+      solution_sample.npy    the solution at DUMP_SAMPLE_POINTS grid points drawn once from a fixed seed, in
+                             row-major order -- the same points in every run with the same --n"""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "residual_history.npy"), np.asarray(hist, dtype=np.float64))
+    if phi.size <= DUMP_SAMPLE_POINTS:
+        np.save(os.path.join(out_dir, "solution.npy"), phi)
+        return
+    idx = np.sort(np.random.default_rng(0).choice(phi.size, DUMP_SAMPLE_POINTS, replace=False))
+    np.save(os.path.join(out_dir, "solution_sample.npy"), phi.reshape(-1)[idx])
+
+
 def sine_rhs(n, out):
     """DynamicGridUtils::compute_rhs with a = p = q = 1, via its separable form (same rounding order:
     (factor * sin(pi x)) * sin(pi y))."""
@@ -454,6 +473,8 @@ def run_single(args):
     ms_per_step = 1e3 * wall / args.steps
     value = n * n / (wall / args.steps) / 1e9
     converged = bool(hist[-1] < REL_TOL * hist[0])
+    if args.dump_outputs:  # before the roofline passes below overwrite the iterate
+        dump_outputs(args.dump_outputs, s.get_solution(), hist)
 
     # ---- roofline of the dominant kernel (level-0 fused passes), timed alone with CUDA events ----
     t_down = s.bench_pass(0, 0, 5)
@@ -565,10 +586,16 @@ def main():
                     help="--impl reference: skip the N=4097 solve measured end to end (~1 min)")
     ap.add_argument("--agglomerate-below", type=int, default=513, dest="agglomerate_below",
                     help="multi-GPU: levels with n <= this run on rank 0 only")
+    ap.add_argument("--dump-outputs", metavar="DIR", dest="dump_outputs",
+                    help="write what the last timed solve returned to DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or world > 1 or args.gpus > 1):
+        ap.error("--dump-outputs is implemented for the CUDA path on one GPU")
     if args.impl == "reference":
         return run_reference(args)
-    world = int(os.environ.get("WORLD_SIZE", "1"))
     if world > 1 or args.gpus > 1:
         import bench_dist
         return bench_dist.run(args)
