@@ -310,6 +310,11 @@ __device__ __forceinline__ void lds_v2(uint32_t a, double &v0, double &v1)
     std::memcpy(&v1, emu_smem + a + 8, 8);
 }
 __device__ __forceinline__ void sts_zero_v2(uint32_t a) { std::memset(emu_smem + a, 0, 16); }
+__device__ __forceinline__ void sts_v2(uint32_t a, double v0, double v1)
+{
+    std::memcpy(emu_smem + a, &v0, 8);
+    std::memcpy(emu_smem + a + 8, &v1, 8);
+}
 __device__ __forceinline__ void publish_epoch(int *flag, int epoch) { *(volatile int *)flag = epoch; }
 __device__ __forceinline__ void __threadfence_system() {}
 __device__ __forceinline__ bool wait_flag(const int *flag, int epoch) { return *(const volatile int *)flag >= epoch; }
@@ -332,6 +337,10 @@ __device__ __forceinline__ void sts_zero_v2(uint32_t a)
 {
     asm volatile("st.shared.v2.f64 [%0], {%1, %1};\n" ::"r"(a), "d"(0.0) : "memory");
 }
+__device__ __forceinline__ void sts_v2(uint32_t a, double v0, double v1)
+{
+    asm volatile("st.shared.v2.f64 [%0], {%1, %2};\n" ::"r"(a), "d"(v0), "d"(v1) : "memory");
+}
 __device__ __forceinline__ void publish_epoch(int *flag, int epoch)
 {
     asm volatile("st.release.sys.global.s32 [%0], %1;" ::"l"(flag), "r"(epoch) : "memory");
@@ -340,7 +349,10 @@ __device__ __forceinline__ void publish_epoch(int *flag, int epoch)
 extern __shared__ __align__(16) unsigned char g_dyn_smem[];
 #endif
 
-template <int C, int PF, int S, bool USE_X>
+// GEN_F (cross-cycle pass on one GPU, analytic right-hand side): f(row, col) = fx[col] * sy[row] is not streamed from HBM
+// but formed when the row is issued -- the same dmul(dmul(factor, sin_x), sin_y) k_rhs_separable wrote, so the same
+// bits -- and stored into the same ring slot with st.shared.  The ring is lane-private: program order is enough.
+template <int C, int PF, int S, bool USE_X, bool GEN_F = false>
 struct SmemFeed {
     static constexpr int UNROLL = 2;
     static constexpr int NF = (PF + S + 2 <= 8) ? 8 : 16;            // f ring slots  (power of two >= PF + S + 2)
@@ -354,12 +366,34 @@ struct SmemFeed {
     const double *x, *f;
     RowSource src;
     int pitch, last_row, t;
+    double fx[C];           // GEN_F: fx of this lane's columns
+    const double *sy;       // GEN_F: sy[row], rows [-PADY, ny + PADY)
+    double sy_next;         // GEN_F: sy of the row the next issue() fills (rows are issued in order)
+    // GEN_F: call before init().  fx addresses logical column 0 of a padded row, sy logical row 0.
+    __device__ __forceinline__ void set_rhs_tables(const double *fx_, const double *sy_, int col)
+    {
+#pragma unroll
+        for (int p = 0; p < PLANES; ++p) {
+            const double2 a = __ldg(reinterpret_cast<const double2 *>(fx_ + col) + p);
+            fx[2 * p] = a.x;
+            fx[2 * p + 1] = a.y;
+        }
+        sy = sy_;
+    }
     __device__ __forceinline__ void issue(int row, int slot_t)
     {
-        const double *fr = src.f_row(f, row);
         uint32_t fa = fbase + (uint32_t)(slot_t & (NF - 1)) * ROW_BYTES;
+        if constexpr (GEN_F) {
+            // issued rows are consecutive (clamped at last_row): fetch sy one row ahead so no store waits for a load
+            const double syr = sy_next;
+            sy_next = __ldg(sy + min(row + 1, last_row));
 #pragma unroll
-        for (int p = 0; p < PLANES; ++p) cp_async16(fa + p * 512, fr + 2 * p);
+            for (int p = 0; p < PLANES; ++p) sts_v2(fa + p * 512, dmul(fx[2 * p], syr), dmul(fx[2 * p + 1], syr));
+        } else {
+            const double *fr = src.f_row(f, row);
+#pragma unroll
+            for (int p = 0; p < PLANES; ++p) cp_async16(fa + p * 512, fr + 2 * p);
+        }
         if (USE_X) {
             const double *xr = src.x_row(x, row);
             uint32_t xa = xbase + (uint32_t)(slot_t & (NXR - 1)) * ROW_BYTES;
@@ -392,6 +426,7 @@ struct SmemFeed {
             for (int p = 0; p < PLANES; ++p) sts_zero_v2(base + sl * ROW_BYTES + p * 512 + lane * 16);
         fbase = base + lane * 16;
         xbase = base + NF * ROW_BYTES + lane * 16;
+        if constexpr (GEN_F) sy_next = __ldg(sy + j_start);
 #pragma unroll
         for (int d = 0; d < PF; ++d) issue(j_start + d, d);
     }
@@ -788,15 +823,18 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
 //     not survive; x_k is written every cycle instead (the pass of the next cycle honours `done` and leaves it alone).
 // Same arithmetic, same order as the two passes: every value is bit-identical.  On row slabs (several GPUs) the input's halo rows -- 6 above, 4 below -- are copied from the
 // neighbours' arrays in the halo prologue, exactly as Pass A does for the iterate.
+//   * GEN_F (one GPU, f written by pmg_set_rhs_sine): f is not read; the row feed forms f = fx[col] * sy[row] from two
+//     padded tables (SmemFeed), 20 B/point instead of 28.  Every stage of the row pipeline is the same code.
 // ---------------------------------------------------------------------------------------------------
-template <int C, int PF, int MINB, int S2, int S1, bool WEIGHTED>
+template <int C, int PF, int MINB, int S2, int S1, bool WEIGHTED, bool GEN_F = false>
 __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
     k_cross(const double *__restrict__ xb, double *__restrict__ xo, double *__restrict__ xk, const double *__restrict__ f,
             const double *__restrict__ e, double *__restrict__ cf, StripGeom g, int pitch_c, int lo, int nc, JacobiCoef coef,
-            double inv_h2, double *__restrict__ partials, const int *__restrict__ done, HaloPeers hp)
+            double inv_h2, double *__restrict__ partials, const int *__restrict__ done, HaloPeers hp,
+            const double *__restrict__ rhs_fx, const double *__restrict__ rhs_sy)
 {
     constexpr int S = S2 + S1;
-    using Feed = SmemFeed<C, PF, S, true>;
+    using Feed = SmemFeed<C, PF, S, true, GEN_F>;
     pdl_wait();
     if (done != nullptr && *done) return;
     static_assert(Feed::UNROLL % 2 == 0, "rows are processed in (even, odd) pairs");
@@ -858,6 +896,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
         }
     }
     Feed feed;
+    if constexpr (GEN_F) feed.set_rhs_tables(rhs_fx, rhs_sy, col);
     feed.init(xb, f, g.pitch, col, j_start, g.ny + PADY - 1, lane, threadIdx.x >> 5, HaloPeers{}, g.ny);
 
     const int cc = col >> 1;
@@ -1219,7 +1258,7 @@ void up_launch(const FusedLevel &lv, const double *e, int pitch_c, double omega,
 }
 
 // geometry of the cross-cycle pass: 4 sweeps + residual + restriction eat 6 columns per side
-template <int C, int PF, int MINB, bool WEIGHTED>
+template <int C, int PF, int MINB, bool WEIGHTED, bool GEN_F = false>
 void cross_launch_w(const FusedLevel &lv_in, double *xb_out, const double *e, int pitch_c, double *cf, int lo, double *d_partials,
                     int *n_partials, const JacobiCoef &c, const int *done, cudaStream_t st)
 {
@@ -1229,11 +1268,11 @@ void cross_launch_w(const FusedLevel &lv_in, double *xb_out, const double *e, in
     StripGeom g = make_geom(lv_in, 6, v, 0, 0, C == 2 ? 6 : 8);
     double inv = 1.0 / (lv_in.h * lv_in.h);
     int nc = (lv_in.n - 1) / 2 + 1;
-    auto k = k_cross<C, PF, MINB, 2, 2, WEIGHTED>;
-    int sm = WARPS_PER_CTA * SmemFeed<C, PF, 4, true>::SMEM_PER_WARP;
+    auto k = k_cross<C, PF, MINB, 2, 2, WEIGHTED, GEN_F>;
+    int sm = WARPS_PER_CTA * SmemFeed<C, PF, 4, true, GEN_F>::SMEM_PER_WARP;
     PMG_SMEM_ONCE(k, sm);
     PMG_LAUNCH(k, dim3(grid_for(g)), dim3(32 * WARPS_PER_CTA), sm, st, lv_in.xb, xb_out, lv_in.x, lv_in.f, e, cf, g, pitch_c, lo, nc, c,
-               inv, d_partials, done, lv_in.hp);
+               inv, d_partials, done, lv_in.hp, lv_in.rhs_fx, lv_in.rhs_sy);
     if (n_partials) *n_partials = g.n_strips * g.n_chunks;
 }
 
@@ -1280,6 +1319,8 @@ void launch_fused_cross(const FusedLevel &lv, double *xb_out, const double *coar
 {
     const int lo = prolong_mode == PMG_PROLONG_FULL ? 1 : 2;
     JacobiCoef c = jacobi_coef(lv.h, omega);
+    // f from the tables: one GPU only (a slab's halo rows of f are not generated), and only when the caller passed them
+    const bool gen_f = lv.rhs_fx != nullptr && lv.rhs_sy != nullptr && lv.ny == 0;
 #define PMG_CROSS(MINB)                                                                                                        \
     do {                                                                                                                       \
         if (c.weighted)                                                                                                        \
@@ -1297,7 +1338,12 @@ void launch_fused_cross(const FusedLevel &lv, double *xb_out, const double *coar
         else                                                                                                                   \
             cross_launch_w<4, PF, 2, false>(lv, xb_out, coarse_x, pitch_c, coarse_f, lo, d_partials, n_partials, c, done, st);  \
     } while (0)
-        if (g_cross_minb == 2)
+        if (g_cross_minb == 2 && gen_f) {  // the default shape alone has the generated-f flavour
+            if (c.weighted)
+                cross_launch_w<4, 2, 2, true, true>(lv, xb_out, coarse_x, pitch_c, coarse_f, lo, d_partials, n_partials, c, done, st);
+            else
+                cross_launch_w<4, 2, 2, false, true>(lv, xb_out, coarse_x, pitch_c, coarse_f, lo, d_partials, n_partials, c, done, st);
+        } else if (g_cross_minb == 2)
             PMG_CROSS4(2);
         else
             PMG_CROSS4(3);

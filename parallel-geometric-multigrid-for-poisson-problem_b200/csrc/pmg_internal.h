@@ -306,6 +306,10 @@ struct FusedLevel {
     int ny, yoff, ext_lo, ext_hi;
     int span_lo, span_hi;  // if span_hi > span_lo: write only local rows [span_lo, span_hi) (span_lo even)
     HaloPeers hp;          // Pass A only: fused halo exchange (wait for the neighbours, read their rows in place)
+    // (nullable; cross-cycle pass, one GPU) f is separable and bit for bit f(y, x) = fx[x] * sy[y] with zeros in the padding:
+    // fx addresses logical column 0 of one padded row (pitch doubles), sy logical row 0 of n + 2*PADY entries.  The
+    // default shape then forms f in the pass instead of reading it (20 B/point instead of 28).
+    const double *rhs_fx, *rhs_sy;
 };
 // Pass A (down): xb = S^nu1(x);  coarse_f(interior) = R(f - A xb).  x_is_zero: the iterate is known to
 // be identically zero on entry (coarse levels of a V-cycle) so x is not read.
@@ -328,7 +332,7 @@ void launch_fused_up(const FusedLevel &lv, const double *coarse_x, int pitch_c, 
 int fused_max_partials(int n);
 // Cross-cycle pass (level 0 of a V-cycle solve, one GPU): Pass B of cycle k and Pass A of cycle k+1 in one sweep over
 // HBM -- reads lv.xb (xb_k), coarse_x (e_k), lv.f; writes lv.x (x_k), xb_out (xb_{k+1}, NOT lv.xb), coarse_f and the partial
-// sums of the residual norm of x_k.  36 B/point instead of 52.  Row slabs: lv.hp = the neighbours' copies of the INPUT array
+// sums of the residual norm of x_k.  36 B/point instead of 52 (28 without x_k; 20 when f comes from lv.rhs_fx / rhs_sy).  Row slabs: lv.hp = the neighbours' copies of the INPUT array
 // (x_up / x_dn / x_keep / flags / epoch as for Pass A); rows [0, ny) are written, 6 halo rows above and 4 below are read.
 bool fused_cross_supported(int nu1, int nu2);
 double fused_cross_utilisation(int n, int rows);  // resident warp slots the pass fills (the solve wants >= 0.9)

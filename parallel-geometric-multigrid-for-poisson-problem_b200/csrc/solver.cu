@@ -101,7 +101,12 @@ struct pmg_solver {
     // F-cycle: level-0 analytic RHS lives in its own array so the caller's f survives
     double *base_f_fmg0 = nullptr, *f_fmg0 = nullptr;
     bool fmg_ready = false;
-    bool rhs_is_analytic = false;  // level 0's f was written by pmg_set_rhs_sine and by nothing since (one GPU)
+    bool rhs_is_analytic = false;  // level 0's f was written by pmg_set_rhs_sine and by nothing since (one GPU); change it
+                                   // with set_rhs_analytic (the cross-cycle graphs depend on it)
+    // level 0's analytic right-hand side as f(y, x) = fx[x] * sy[y] (FusedLevel::rhs_fx / rhs_sy), built by pmg_set_rhs_sine:
+    // the cross-cycle pass forms f from these instead of reading it while rhs_is_analytic holds for the array rhs_tab_f
+    double *base_rhs_fx = nullptr, *base_rhs_sy = nullptr;
+    const double *rhs_fx = nullptr, *rhs_sy = nullptr, *rhs_tab_f = nullptr;
     bool fmg0_rhs_cached = false;  // f_fmg0 holds the analytic right-hand side of level 0 (a constant of the hierarchy)
     // CUDA graphs of one fused cycle, keyed by [kind V/W][0: no norm, 1: norm -> d_scalar,
     // 2: norm -> device-side solve control (asynchronous solve)]
@@ -182,6 +187,15 @@ struct pmg_solver {
 
 namespace pmg {
 
+static void drop_cross_graphs(pmg_solver *s)
+{
+    for (auto &g : s->cross_graph)
+        if (g) {
+            cudaGraphExecDestroy(g);
+            g = nullptr;
+        }
+}
+
 static void drop_graphs(pmg_solver *s)
 {
     for (auto &row : s->graph)
@@ -200,11 +214,15 @@ static void drop_graphs(pmg_solver *s)
             cudaGraphExecDestroy(g);
             g = nullptr;
         }
-    for (auto &g : s->cross_graph)
-        if (g) {
-            cudaGraphExecDestroy(g);
-            g = nullptr;
-        }
+    drop_cross_graphs(s);
+}
+
+// A captured cross-cycle graph keeps the f feed it was captured with (generated from the tables or read from HBM): a graph
+// captured after pmg_set_rhs_sine must not outlive a user right-hand side, so the graphs go whenever the flag changes.
+static void set_rhs_analytic(pmg_solver *s, bool on)
+{
+    if (s->rhs_is_analytic != on) drop_cross_graphs(s);
+    s->rhs_is_analytic = on;
 }
 
 static FusedLevel fused_view(const Level &L)
@@ -221,7 +239,18 @@ static FusedLevel fused_view(const Level &L)
     v.ext_lo = v.ext_hi = 0;
     v.span_lo = v.span_hi = 0;
     v.hp = HaloPeers{};
+    v.rhs_fx = v.rhs_sy = nullptr;
     return v;
+}
+
+// The cross-cycle pass on level 0 with f generated from the tables -- only if v.f is the array pmg_set_rhs_sine wrote and
+// nothing has written since (PCG and the F-cycle point level 0 at other arrays for a while)
+static void use_rhs_tables(const pmg_solver *s, FusedLevel &v)
+{
+    if (s->rhs_is_analytic && s->rhs_fx != nullptr && v.f == s->rhs_tab_f) {
+        v.rhs_fx = s->rhs_fx;
+        v.rhs_sy = s->rhs_sy;
+    }
 }
 
 static pmg_status alloc_zero(double **p, size_t elems)
@@ -1521,6 +1550,8 @@ void pmg_destroy(pmg_solver *s)
         cudaFree(L.base_r);
         cudaFree(L.d_sin);
     }
+    cudaFree(s->base_rhs_fx);
+    cudaFree(s->base_rhs_sy);
     cudaFree(s->base_f_fmg0);
     for (double *b : s->pcg_base) cudaFree(b);
     cudaFree(s->base_xc);
@@ -1585,7 +1616,7 @@ static pmg_status copy_in(pmg_solver *s, double *dst_logical, const double *src,
 
 pmg_status pmg_set_rhs(pmg_solver *s, const double *f, pmg_mem where)
 {
-    if (s) s->rhs_is_analytic = false;
+    if (s) set_rhs_analytic(s, false);
     return copy_in(s, s ? s->lv[0].f : nullptr, f, where);
 }
 
@@ -1657,7 +1688,7 @@ pmg_status pmg_commit_rhs(pmg_solver *s)
     PMG_CUDA(cudaStreamWaitEvent(s->stream, s->ev_staged, 0));
     // a device copy (1.4 ms at N = 16385) rather than a pointer swap: the captured cycle graphs and, on several GPUs,
     // the neighbours' peer mappings keep addressing the same f array
-    s->rhs_is_analytic = false;
+    set_rhs_analytic(s, false);
     PMG_CUDA(cudaMemcpyAsync(L.base_f, s->base_f_stage, L.elems * sizeof(double), cudaMemcpyDeviceToDevice, s->stream));
     PMG_CUDA(cudaEventRecord(s->ev_consumed, s->stream));
     s->staged = false;
@@ -1697,6 +1728,34 @@ pmg_status pmg_fetch_solution_wait(pmg_solver *s)
     return PMG_OK;
 }
 
+// fx = factor * sin in the padded column layout of level 0, sy = sin with PADY zero rows above and below: dmul(fx[x], sy[y])
+// is the dmul(dmul(factor, sin_x), sin_y) k_rhs_separable writes, and +0 wherever the array holds its zero padding -- as long
+// as no sine value carries a sign bit (-0 * +0 would give -0).  If one does, no tables are built and the pass reads f.
+static pmg_status ensure_rhs_tables(pmg_solver *s)
+{
+    if (s->base_rhs_fx != nullptr) return PMG_OK;
+    const Level &L = s->lv[0];
+    std::vector<double> sn(L.n);
+    PMG_CUDA(cudaMemcpy(sn.data(), L.d_sin, L.n * sizeof(double), cudaMemcpyDeviceToHost));
+    for (double v : sn)
+        if (std::signbit(v)) return PMG_OK;
+    const double a = 1.0, p = 1.0, q = 1.0;
+    const double factor = (M_PI * M_PI / (a * a)) * (p * p + q * q);  // as analytic_rhs
+    std::vector<double> fx(L.pitch, 0.0), sy(L.n + 2 * PADY, 0.0);
+    for (int i = 0; i < L.n; ++i) {
+        fx[PADX + i] = factor * sn[i];
+        sy[PADY + i] = sn[i];
+    }
+    pmg_status rc = alloc_zero(&s->base_rhs_fx, fx.size());
+    if (rc == PMG_OK) rc = alloc_zero(&s->base_rhs_sy, sy.size());
+    if (rc != PMG_OK) return rc;
+    PMG_CUDA(cudaMemcpy(s->base_rhs_fx, fx.data(), fx.size() * sizeof(double), cudaMemcpyHostToDevice));
+    PMG_CUDA(cudaMemcpy(s->base_rhs_sy, sy.data(), sy.size() * sizeof(double), cudaMemcpyHostToDevice));
+    s->rhs_fx = s->base_rhs_fx + PADX;
+    s->rhs_sy = s->base_rhs_sy + PADY;
+    return PMG_OK;
+}
+
 pmg_status pmg_set_rhs_sine(pmg_solver *s)
 {
     if (!s) return fail(PMG_ERR_INVALID, "null argument");
@@ -1712,7 +1771,9 @@ pmg_status pmg_set_rhs_sine(pmg_solver *s)
                              L.d_sin + ga, s->stream);
     } else {
         analytic_rhs(s, s->lv[0], s->lv[0].f);
-        s->rhs_is_analytic = true;
+        if ((rc = ensure_rhs_tables(s)) != PMG_OK) return rc;
+        s->rhs_tab_f = s->lv[0].f;
+        set_rhs_analytic(s, true);
     }
     PMG_CUDA(cudaStreamSynchronize(s->stream));
     PMG_CUDA(cudaGetLastError());
@@ -1979,6 +2040,7 @@ static pmg_status run_cross_cycle(pmg_solver *s, int parity)
         FusedLevel v = fused_view(L);
         v.x = nullptr;                            // x_k is not written (solve_cross produces it once, at the end)
         v.xb = parity ? s->xc : L.xb;             // input: xb_k
+        use_rhs_tables(s, v);                     // f generated in the pass (set_rhs_analytic drops this graph when that changes)
         double *out = parity ? L.xb : s->xc;      // output: xb_{k+1}
         launch_fused_cross(v, out, K.x, K.f, K.pitch, c.omega, c.prolong_mode, s->d_partials, &np, s->stream, done);
         launch_cycle_finish(s->d_partials, np, s->d_ctrl, s->d_hist2, s->stream);
@@ -2391,6 +2453,7 @@ pmg_status pmg_bench_pass(pmg_solver *s, int which, int level, int reps, double 
         if (which == 4) {
             FusedLevel v = fused_view(L);
             v.x = nullptr;
+            use_rhs_tables(s, v);  // the flavour pmg_solve runs
             launch_fused_cross(v, s->xc, K.x, K.f, K.pitch, c.omega, c.prolong_mode, s->d_partials, &np, s->stream);
         } else if (which == 0 || which == 3)
             launch_fused_down(fused_view(L), K.f, K.pitch, c.nu1, c.omega, which == 3, s->stream);
