@@ -97,6 +97,45 @@ __device__ __forceinline__ void store_row(double *__restrict__ p, const Row<C> &
     }
 }
 
+// an owner lane's row: all C columns, or (the lane whose slot 0 is the last column, wide cross pass) the first one only.
+// Both as predicated stores: a branch around each would cost more instructions in the row loop than the stores themselves.
+template <int C>
+__device__ __forceinline__ void store_owned(double *__restrict__ p, const Row<C> &r, bool all, bool first_only)
+{
+#ifndef PMG_HOST_EMULATION
+    if constexpr (C == 4) {
+        asm volatile("{\n\t.reg .pred pa, po;\n\tsetp.ne.b32 pa, %5, 0;\n\tsetp.ne.b32 po, %6, 0;\n\t"
+                     "@pa st.global.v4.f64 [%0], {%1, %2, %3, %4};\n\t@po st.global.f64 [%0], %1;\n\t}"
+                     ::"l"(p), "d"(r.v[0]), "d"(r.v[1]), "d"(r.v[2]), "d"(r.v[3]), "r"((int)all), "r"((int)first_only)
+                     : "memory");
+        return;
+    }
+#endif
+    if (all)
+        store_row<C>(p, r);
+    else if (first_only)
+        *p = r.v[0];
+}
+
+// coarse points of a lane (C / 2 of them): all, or the first one only
+template <int NP>
+__device__ __forceinline__ void store_coarse_owned(double *__restrict__ p, const double (&o)[NP], bool all, bool first_only)
+{
+#ifndef PMG_HOST_EMULATION
+    if constexpr (NP == 2) {
+        asm volatile("{\n\t.reg .pred pa, po;\n\tsetp.ne.b32 pa, %3, 0;\n\tsetp.ne.b32 po, %4, 0;\n\t"
+                     "@pa st.global.v2.f64 [%0], {%1, %2};\n\t@po st.global.f64 [%0], %1;\n\t}"
+                     ::"l"(p), "d"(o[0]), "d"(o[1]), "r"((int)all), "r"((int)first_only)
+                     : "memory");
+        return;
+    }
+#endif
+    if (NP == 2 && all)
+        *reinterpret_cast<double2 *>(p) = make_double2(o[0], o[NP - 1]);
+    else if (NP == 1 ? all : first_only)
+        *p = o[0];
+}
+
 template <int C>
 __device__ __forceinline__ Row<C> zero_row()
 {
@@ -156,6 +195,28 @@ struct SweepStage {
 #pragma unroll
         for (int k = 0; k < C; ++k)
             part.v[k] = dadd(dadd(dadd(dmul(c.h2, f_row.v[k]), w.v[k]), e.v[k]), prev.v[k]);
+        cen[p ^ 1] = in;
+        return out;
+    }
+    // The same stage on the wide cross-pass geometry (k_cross, 4 columns per lane): `h2f` = h^2 f of row i, formed once by
+    // the feed.  Only slot 0 can hold a Dirichlet column, so slots 1-3 are frozen only with the whole row: keep0 = slot 0
+    // keeps its value, keep_row = the whole output row does (a constant false where the row's parity rules it out).
+    template <bool WEIGHTED>
+    __device__ __forceinline__ Row<C> step_wide(const int p, const Row<C> &in, const Row<C> &h2f, const JacobiCoef &c,
+                                                bool keep0, bool keep_row)
+    {
+        static_assert(C == 4, "wide geometry: 4 columns per lane");
+        Row<C> out, w, e;
+        const Row<C> &prev = cen[p];
+#pragma unroll
+        for (int k = 0; k < C; ++k) {
+            const double sum = dadd(part.v[k], in.v[k]);
+            double val = WEIGHTED ? dadd(dmul(c.om1, prev.v[k]), dmul(c.w4, sum)) : dmul(0.25, sum);
+            out.v[k] = ((k == 0) ? keep0 : keep_row) ? prev.v[k] : val;
+        }
+        neighbours<C>(in, w, e);
+#pragma unroll
+        for (int k = 0; k < C; ++k) part.v[k] = dadd(dadd(dadd(h2f.v[k], w.v[k]), e.v[k]), prev.v[k]);
         cen[p ^ 1] = in;
         return out;
     }
@@ -352,20 +413,24 @@ extern __shared__ __align__(16) unsigned char g_dyn_smem[];
 // GEN_F (cross-cycle pass on one GPU, analytic right-hand side): f(row, col) = fx[col] * sy[row] is not streamed from HBM
 // but formed when the row is issued -- the same dmul(dmul(factor, sin_x), sin_y) k_rhs_separable wrote, so the same
 // bits -- and stored into the same ring slot with st.shared.  The ring is lane-private: program order is enough.
-template <int C, int PF, int S, bool USE_X, bool GEN_F = false>
+// H2F: a second ring of NF slots, parallel to the f ring, holds h^2 f of the same rows, formed once per point (with GEN_F
+// when the row is generated, otherwise when its cp.async has landed) instead of once per sweep stage that reads it.
+template <int C, int PF, int S, bool USE_X, bool GEN_F = false, bool H2F = false>
 struct SmemFeed {
     static constexpr int UNROLL = 2;
     static constexpr int NF = (PF + S + 2 <= 8) ? 8 : 16;            // f ring slots  (power of two >= PF + S + 2)
     static constexpr int NXR = (PF + 1 <= 4) ? 4 : 8;                // x ring slots  (power of two >= PF + 1)
     static constexpr int NX = USE_X ? NXR : 0;
+    static constexpr int NH = H2F ? NF : 0;                          // h^2 f ring slots (slot i holds the row of f slot i)
     static constexpr int PLANES = C / 2;               // 16-byte pieces per lane per row
     static constexpr int ROW_BYTES = PLANES * 512;     // plane p of a row: 32 lanes x 16 B, conflict free
-    static constexpr int SMEM_PER_WARP = (NF + NX) * ROW_BYTES;
+    static constexpr int SMEM_PER_WARP = (NF + NH + NX) * ROW_BYTES;
     static_assert(PF + S + 2 <= NF && PF + 1 <= NXR, "ring too small");
-    uint32_t fbase, xbase;  // shared-window addresses of this lane's first piece in slot 0
+    uint32_t fbase, xbase;  // shared-window addresses of this lane's first piece in slot 0 (h^2 f ring: fbase + NF rows)
     const double *x, *f;
     RowSource src;
     int pitch, last_row, t;
+    double h2;              // H2F
     double fx[C];           // GEN_F: fx of this lane's columns
     const double *sy;       // GEN_F: sy[row], rows [-PADY, ny + PADY)
     double sy_next;         // GEN_F: sy of the row the next issue() fills (rows are issued in order)
@@ -388,7 +453,11 @@ struct SmemFeed {
             const double syr = sy_next;
             sy_next = __ldg(sy + min(row + 1, last_row));
 #pragma unroll
-            for (int p = 0; p < PLANES; ++p) sts_v2(fa + p * 512, dmul(fx[2 * p], syr), dmul(fx[2 * p + 1], syr));
+            for (int p = 0; p < PLANES; ++p) {
+                const double f0 = dmul(fx[2 * p], syr), f1 = dmul(fx[2 * p + 1], syr);
+                sts_v2(fa + p * 512, f0, f1);
+                if constexpr (H2F) sts_v2(fa + NF * ROW_BYTES + p * 512, dmul(h2, f0), dmul(h2, f1));
+            }
         } else {
             const double *fr = src.f_row(f, row);
 #pragma unroll
@@ -421,11 +490,11 @@ struct SmemFeed {
         uint32_t base = (uint32_t)__cvta_generic_to_shared(g_dyn_smem) + warp_in_cta * SMEM_PER_WARP;
         // zero this lane's pieces (warm-up steps read slots that were never filled)
 #pragma unroll
-        for (int sl = 0; sl < NF + NX; ++sl)
+        for (int sl = 0; sl < NF + NH + NX; ++sl)
 #pragma unroll
             for (int p = 0; p < PLANES; ++p) sts_zero_v2(base + sl * ROW_BYTES + p * 512 + lane * 16);
         fbase = base + lane * 16;
-        xbase = base + NF * ROW_BYTES + lane * 16;
+        xbase = base + (NF + NH) * ROW_BYTES + lane * 16;
         if constexpr (GEN_F) sy_next = __ldg(sy + j_start);
 #pragma unroll
         for (int d = 0; d < PF; ++d) issue(j_start + d, d);
@@ -434,6 +503,12 @@ struct SmemFeed {
     {
         cp_async_wait<PF - 1>();  // all but the newest PF-1 groups have landed => row jj is in its slot
         if (src.keeps(jj)) store_row<C>(src.f_keep + (ptrdiff_t)jj * pitch, lds_row(fbase + (uint32_t)(t & (NF - 1)) * ROW_BYTES));
+        if constexpr (H2F && !GEN_F) {
+            const uint32_t fa = fbase + (uint32_t)(t & (NF - 1)) * ROW_BYTES;
+            const Row<C> fr = lds_row(fa);
+#pragma unroll
+            for (int p = 0; p < PLANES; ++p) sts_v2(fa + NF * ROW_BYTES + p * 512, dmul(h2, fr.v[2 * p]), dmul(h2, fr.v[2 * p + 1]));
+        }
         Row<C> cur = USE_X ? lds_row(xbase + (uint32_t)(t & (NXR - 1)) * ROW_BYTES) : zero_row<C>();
         issue(min(jj + PF, last_row), t + PF);
         return cur;
@@ -441,6 +516,10 @@ struct SmemFeed {
     __device__ __forceinline__ Row<C> f_row(int d) const
     {
         return lds_row(fbase + (uint32_t)((t - d) & (NF - 1)) * ROW_BYTES);
+    }
+    __device__ __forceinline__ Row<C> h2f_row(int d) const  // H2F: h^2 f of row jj - d
+    {
+        return lds_row(fbase + (uint32_t)(NF + ((t - d) & (NF - 1))) * ROW_BYTES);
     }
     __device__ __forceinline__ void end() { ++t; }
 };
@@ -834,7 +913,25 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
             const double *__restrict__ rhs_fx, const double *__restrict__ rhs_sy)
 {
     constexpr int S = S2 + S1;
-    using Feed = SmemFeed<C, PF, S, true, GEN_F>;
+    // WIDE: 4 columns per lane on strips of 128 columns that own 112 (halo 8), so col = -8 + 112 strip + 4 lane = 0 (mod 4);
+    // every level has n = 2^k + 1 with n - 1 = 0 (mod 4) (launch_fused_cross takes a narrow shape for n = 3).  Hence the
+    // Dirichlet columns 0 and n - 1 can only sit in slot 0 of a lane; slots 1-3 hold interior columns or padding.  The
+    // wide pass freezes slot 0 only and lets the padding columns (and the padding rows of odd parity) compute values that
+    // are never read by a domain point:
+    //  * a sweep stage's output at a point depends on the input at that point and at its 4 neighbours, unless the point is
+    //    frozen -- then it is its input.  Columns 0 and n - 1 are frozen in every stage, rows 0 and n - 1 (both even) in
+    //    every stage whose output row is even.  A padding column's only domain neighbours are column 0 or n - 1, a padding
+    //    row's only domain neighbours are row 0 or n - 1; by induction over the stages every domain value of every stage
+    //    equals the value with zero padding.  The prolongation's corrections in padding slots are input to such columns.
+    //  * residual: r at an interior point reads x at domain points only.  r at a boundary or padding point is read by the
+    //    norm, which masks it per lane (nmask) and per row, and by the restriction only for coarse boundary or padding
+    //    columns (coarse point ic reads fine columns 2ic - 1 .. 2ic + 1; for 1 <= ic <= nc - 2, including the west value
+    //    shuffled from the lane to the left, that is [1, n - 2]; likewise rows).  Coarse columns 0 and nc - 1 = (n - 1) / 2
+    //    are even, i.e. q = 0, and are still set to 0.
+    //  * stores: owner lanes start at column 0; a lane beyond column n - 1 stores nothing, the lane at column n - 1 only
+    //    slot 0 (coarse: q = 0).  So the padding of every output array stays zero in HBM (DESIGN section 3).
+    constexpr bool WIDE = (C == 4);
+    using Feed = SmemFeed<C, PF, S, true, GEN_F, WIDE>;
     pdl_wait();
     if (done != nullptr && *done) return;
     static_assert(Feed::UNROLL % 2 == 0, "rows are processed in (even, odd) pairs");
@@ -845,6 +942,12 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
     int col, r0, r1;
     bool owner, cin[C];
     strip_setup<C>(g, wid, lane, col, r0, r1, owner, cin);
+    const bool keep_c0 = !cin[0];                                 // WIDE: slot 0 is column 0, n - 1 or padding
+    const bool st_all = owner && (!WIDE || col + C - 1 <= g.n - 1);  // the lane stores all its columns
+    const bool st_one = WIDE && owner && col == g.n - 1;          // ... or only slot 0 (coarse: q = 0)
+    bool nmask[C];                                                // the norm's columns
+#pragma unroll
+    for (int k = 0; k < C; ++k) nmask[k] = owner && cin[k];
 
     // rows this chunk must finish: xb' on [r0, r1) and, for the coarse rows it owns, r' on [2jc-1, 2jc+1]
     int j_start = min(r0, max(r0, 0) - 2) - S;
@@ -861,9 +964,11 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
     double s_mid[NP], s_cor[NP], c_mid[NP], c_ew[NP];
 #pragma unroll
     for (int q = 0; q < NP; ++q) s_mid[q] = s_cor[q] = c_mid[q] = c_ew[q] = 0.0;
+    // columns that receive a correction.  WIDE: slot 2 holds columns 2 .. n - 3 or padding, slot 3 columns 3 .. n - 2 or
+    // padding, so only slots 0 (columns 0, n - 1) and 1 (column 1, skipped by the reference prolongation) need the test
     bool cprol[C];
 #pragma unroll
-    for (int k = 0; k < C; ++k) cprol[k] = (col + k >= lo) && (col + k <= g.n - 2);
+    for (int k = 0; k < C; ++k) cprol[k] = (WIDE && k >= 2) || ((col + k >= lo) && (col + k <= g.n - 2));
 
     // row slabs: tell the neighbours that my rows of the input array are final, then copy their boundary rows into my
     // halo rows (halo prologue: only the warps whose rows reach into a neighbour's slab wait for its flag)
@@ -896,6 +1001,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
         }
     }
     Feed feed;
+    feed.h2 = coef.h2;
     if constexpr (GEN_F) feed.set_rhs_tables(rhs_fx, rhs_sy, col);
     feed.init(xb, f, g.pitch, col, j_start, g.ny + PADY - 1, lane, threadIdx.x >> 5, HaloPeers{}, g.ny);
 
@@ -927,7 +1033,8 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
             const int jj = j + u;  // u even: fine row 2jc, u odd: 2jc+1
             Row<C> cur = feed.begin(u, jj);
             {   // prolongation-and-add (MultiGrid.hpp:86)
-                const bool rowp = (jj + g.yoff >= lo) && (jj + g.yoff <= g.n - 2);
+                // an odd row below n - 1 is at most n - 2 (n is odd): odd rows need the lower bound only
+                const bool rowp = (jj + g.yoff >= lo) && ((u & 1) != 0 || jj + g.yoff <= g.n - 2);
                 double corr[C];  // the coarse values each point interpolates, summed but not yet weighted
                 if ((u & 1) == 0) {
                     en = eq[0];
@@ -953,38 +1060,49 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
                 for (int k = 0; k < C; ++k)
                     if (rowp && cprol[k]) cur.v[k] = add_correction(cur.v[k], corr[k], u & 1, k & 1);
             }
-            // post-smoothing of cycle k (:89): stage k finishes x row jj-k-1
-#pragma unroll
-            for (int k = 0; k < S2; ++k) {
+            // stage k finishes x row jj-k-1
+            auto sweep = [&](const int k, const Row<C> &in) -> Row<C> {
                 const int out_row = jj - k - 1 + g.yoff;
-                cur = st[k].template step<WEIGHTED>(u & 1, cur, feed.f_row(k), coef, out_row > 0 && out_row < g.n - 1, cin);
-            }
+                const bool interior_row = out_row > 0 && out_row < g.n - 1;
+                if constexpr (WIDE) {
+                    // rows 0 and n - 1 are even (yoff is even): only the stages whose output row is even can meet one
+                    const bool keep_row = ((u + k + 1) & 1) == 0 && !interior_row;
+                    return st[k].template step_wide<WEIGHTED>(u & 1, in, feed.h2f_row(k), coef, keep_c0 || keep_row, keep_row);
+                } else {
+                    return st[k].template step<WEIGHTED>(u & 1, in, feed.f_row(k), coef, interior_row, cin);
+                }
+            };
+            // post-smoothing of cycle k (:89)
+#pragma unroll
+            for (int k = 0; k < S2; ++k) cur = sweep(k, cur);
             {   // cur = x_k row jj - S2: the iterate of cycle k, written for the case that cycle k is the last one
                 const int krow = jj - S2;
-                if (xk != nullptr && owner && krow >= r0 && krow < r1) store_row<C>(xk + (ptrdiff_t)krow * g.pitch + col, cur);
+                if (xk != nullptr) {
+                    const bool row_ok = krow >= r0 && krow < r1;
+                    store_owned<C>(xk + (ptrdiff_t)krow * g.pitch + col, cur, row_ok && st_all, row_ok && st_one);
+                }
                 // the runner's residual norm of cycle k (MultiGridTestRunner.hpp:210-211): r of x row jj - S2 - 1
                 Row<C> r = rs_norm.step(u & 1, cur, feed.f_row(S2 + 1), inv_h2);
                 const int rrow = jj - S2 - 1;
-                if (owner && rrow >= r0 && rrow < r1 && rrow >= 0 && rrow < g.ny && rrow + g.yoff > 0 &&
-                    rrow + g.yoff < g.n - 1) {
+                // rows 0 and n - 1 are even: an odd row in [r0, r1) is an interior row
+                if (rrow >= r0 && rrow < r1 && rrow >= 0 && rrow < g.ny &&
+                    (((u + S2 + 1) & 1) != 0 || (rrow + g.yoff > 0 && rrow + g.yoff < g.n - 1))) {
 #pragma unroll
                     for (int k = 0; k < C; ++k)
-                        if (cin[k]) acc = dadd(acc, dmul(r.v[k], r.v[k]));
+                        if (nmask[k]) acc = dadd(acc, dmul(r.v[k], r.v[k]));
                 }
             }
             // pre-smoothing of cycle k+1 (:66)
 #pragma unroll
-            for (int k = S2; k < S; ++k) {
-                const int out_row = jj - k - 1 + g.yoff;
-                cur = st[k].template step<WEIGHTED>(u & 1, cur, feed.f_row(k), coef, out_row > 0 && out_row < g.n - 1, cin);
-            }
+            for (int k = S2; k < S; ++k) cur = sweep(k, cur);
             const int xrow = jj - S;
-            if (owner && xrow >= r0 && xrow < r1) store_row<C>(xo + (ptrdiff_t)xrow * g.pitch + col, cur);
+            const bool xrow_ok = xrow >= r0 && xrow < r1;
+            store_owned<C>(xo + (ptrdiff_t)xrow * g.pitch + col, cur, xrow_ok && st_all, xrow_ok && st_one);
             {   // residual + full weighting of cycle k+1 (:69-78), as in k_down
                 Row<C> r = rs.step(u & 1, cur, feed.f_row(S + 1), inv_h2);
                 const int rrow = jj - S - 1;
                 double left = __shfl_up_sync(0xffffffffu, r.v[C - 1], 1);
-                if (rrow & 1) {
+                if (((u + S + 1) & 1) != 0) {  // rrow odd (j is even)
                     const int jc = (rrow - 1) >> 1;
                     const int ic = col >> 1;
                     double o[NP];
@@ -994,18 +1112,14 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
                         double edge = dadd(dadd(c_ew[q], r.v[2 * q]), s_mid[q]);
                         double corner = dadd(dadd(s_cor[q], west), r.v[2 * q + 1]);
                         double val = dfma_pow2(0.0625, corner, dfma_pow2(0.125, edge, dmul(0.25, c_mid[q])));
-                        o[q] = (ic + q >= 1 && ic + q < nc - 1) ? val : 0.0;
+                        // WIDE: q = 1 is an interior coarse column or padding that is not stored
+                        o[q] = ((WIDE && q == 1) || (ic + q >= 1 && ic + q < nc - 1)) ? val : 0.0;
                         s_mid[q] = r.v[2 * q];
                         s_cor[q] = dadd(west, r.v[2 * q + 1]);
                     }
-                    if (owner && jc + ycoarse >= 1 && jc + ycoarse < nc - 1 && 2 * jc >= r0 && 2 * jc < r1 && jc >= 0 &&
-                        2 * jc < g.ny) {
-                        double *dst = cf + (ptrdiff_t)jc * pitch_c + ic;
-                        if (NP == 2)
-                            *reinterpret_cast<double2 *>(dst) = make_double2(o[0], o[NP - 1]);
-                        else
-                            *dst = o[0];
-                    }
+                    const bool jc_ok =
+                        jc + ycoarse >= 1 && jc + ycoarse < nc - 1 && 2 * jc >= r0 && 2 * jc < r1 && jc >= 0 && 2 * jc < g.ny;
+                    store_coarse_owned<NP>(cf + (ptrdiff_t)jc * pitch_c + ic, o, jc_ok && st_all, jc_ok && st_one);
                 } else {
 #pragma unroll
                     for (int q = 0; q < NP; ++q) {
@@ -1269,7 +1383,7 @@ void cross_launch_w(const FusedLevel &lv_in, double *xb_out, const double *e, in
     double inv = 1.0 / (lv_in.h * lv_in.h);
     int nc = (lv_in.n - 1) / 2 + 1;
     auto k = k_cross<C, PF, MINB, 2, 2, WEIGHTED, GEN_F>;
-    int sm = WARPS_PER_CTA * SmemFeed<C, PF, 4, true, GEN_F>::SMEM_PER_WARP;
+    int sm = WARPS_PER_CTA * SmemFeed<C, PF, 4, true, GEN_F, C == 4>::SMEM_PER_WARP;
     PMG_SMEM_ONCE(k, sm);
     PMG_LAUNCH(k, dim3(grid_for(g)), dim3(32 * WARPS_PER_CTA), sm, st, lv_in.xb, xb_out, lv_in.x, lv_in.f, e, cf, g, pitch_c, lo, nc, c,
                inv, d_partials, done, lv_in.hp, lv_in.rhs_fx, lv_in.rhs_sy);
@@ -1330,7 +1444,9 @@ void launch_fused_cross(const FusedLevel &lv, double *xb_out, const double *coar
     } while (0)
     if (g_cross_minb == 4)
         PMG_CROSS(4);
-    else if (g_cross_minb == 2 || g_cross_minb == 7) {  // 4 columns per lane, 8 warps per SM; 7 = one more row of prefetch
+    else if ((g_cross_minb == 2 || g_cross_minb == 7) && (lv.n - 1) % 4 == 0) {
+        // 4 columns per lane, 8 warps per SM; 7 = one more row of prefetch.  The wide kernel freezes the Dirichlet columns in
+        // slot 0 only, which needs n - 1 = 0 (mod 4): every level but n = 3, which takes the narrow shape below
 #define PMG_CROSS4(PF)                                                                                                         \
     do {                                                                                                                       \
         if (c.weighted)                                                                                                        \
