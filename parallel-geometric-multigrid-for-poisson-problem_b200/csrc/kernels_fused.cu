@@ -9,6 +9,10 @@
 //                     = prolongation + Smoother::smooth (+ the runner's residual norm)
 //                       (MultiGrid.hpp:86-89, MultiGridTestRunner.hpp:210-211)   26 B / point
 //
+// First visit of a coarse level (x == 0 on entry): Pass A's first sweep is pointwise in f (sweep_row_from_zero: no
+// neighbours, no row of delay).  On whole levels larger than the L2 cache (fused_rebuild_xb) Pass A does not store xb
+// (10 B / point) and Pass B rebuilds xb = S^nu1(0; f) from the f rows it reads anyway (18 B / point): 28 B instead of 44.
+//
 // Execution model (DESIGN.md section 4).  No shared memory, no block barriers: every WARP owns a
 // strip of 128 columns (32 lanes x 4 consecutive columns, two 128-bit loads per lane per row per
 // array) and streams down a chunk of rows.  All stages of the pass are pipelined over the rows in
@@ -221,6 +225,30 @@ struct SweepStage {
         return out;
     }
 };
+
+// The first sweep from x == 0 (first visit of a coarse level), as a per-point expression of f: no shuffles, no state, no
+// row of delay.  SweepStage::step with every input +0 evaluates, in the reference's order,
+//   sum = ((((h^2 f + W) + E) + S) + N) with W = E = S = N = +0,   val = om1 * x + w4 * sum  (x = +0)  or  0.25 * sum.
+// Adding +0 is exact and idempotent except that it turns -0 into +0, so the four additions are one: dadd(h^2 f, +0)
+// (f = -0, or h^2 f underflowing to -0, must give +0 as in the reference).  dmul(om1, +0) is -0 when omega > 1 (om1 < 0)
+// and +0 otherwise; it is kept because it decides the sign of a zero result: -0 + (w4 * sum) is -0 when w4 * sum
+// underflows to -0, +0 + (-0) is +0.  omega = 1 is the unweighted 0.25 * sum.  Frozen points keep their input, +0.
+template <bool WEIGHTED>
+__device__ __forceinline__ double sweep_from_zero(double f, const JacobiCoef &c)
+{
+    const double sum = dadd(dmul(c.h2, f), 0.0);
+    return WEIGHTED ? dadd(dmul(c.om1, 0.0), dmul(c.w4, sum)) : dmul(0.25, sum);
+}
+
+template <int C, bool WEIGHTED>
+__device__ __forceinline__ Row<C> sweep_row_from_zero(const Row<C> &f_row, const JacobiCoef &c, bool row_interior,
+                                                      const bool (&col_interior)[C])
+{
+    Row<C> out;
+#pragma unroll
+    for (int k = 0; k < C; ++k) out.v[k] = (row_interior && col_interior[k]) ? sweep_from_zero<WEIGHTED>(f_row.v[k], c) : 0.0;
+    return out;
+}
 
 // Residual stage: same pipeline shape; returns r of row i-1 given x row i.
 template <int C>
@@ -559,13 +587,21 @@ __device__ __forceinline__ CoarseRow<C> load_coarse(const double *__restrict__ p
 // PIN ("prolong in", one GPU, with ZEROX): the iterate on entry is P e_in -- the bilinear prolongation of a coarse iterate
 // into a zeroed grid (nested iteration, MultiGrid.hpp:161-164) -- formed on the fly from the coarse rows instead of being
 // written by a fill + a prolongation kernel and read back (8 + 18 + 8 B per point less).
-template <int C, int PF, int MINB, bool SM, int S, bool ZEROX, bool RESID, bool WEIGHTED, bool PROLOGUE = false, bool PIN = false>
+// ZEROX without PIN: the first sweep is pointwise (sweep_row_from_zero) on the arriving f row, so the pipeline has S - 1
+// stages of row delay instead of S and the chunk bounds shrink by one row at each end.
+// NO_XB (one GPU, ZEROX): xb is not stored -- Pass B rebuilds it from f (k_up with REBUILD) -- and the pass only reads f
+// and writes the coarse f.
+template <int C, int PF, int MINB, bool SM, int S, bool ZEROX, bool RESID, bool WEIGHTED, bool PROLOGUE = false, bool PIN = false,
+          bool NO_XB = false>
 __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
     k_down(const double *__restrict__ x, double *__restrict__ xo, const double *__restrict__ f,
            double *__restrict__ cf, StripGeom g, int pitch_c, int nc, JacobiCoef coef, double inv_h2,
            const int *__restrict__ done, HaloPeers hp, const double *__restrict__ e_in, int pitch_e, int lo)
 {
     static_assert(!PIN || (ZEROX && SM), "prolong-in: the iterate is not read, shared-memory feed (row pairs)");
+    static_assert(!NO_XB || (ZEROX && RESID && !PIN), "xb is rebuilt by Pass B only on a first visit");
+    constexpr bool PW = ZEROX && !PIN;  // pointwise first sweep
+    constexpr int SD = PW ? S - 1 : S;  // sweep stages with a row of delay
     using Feed = typename FeedSelect<C, PF, S, !ZEROX, SM>::type;
     pdl_wait();
     const bool pdl_early = gridDim.x <= 296u;  // at most two CTAs per SM: a latency-bound level (pmg_internal.h)
@@ -583,11 +619,12 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
 
     // Rows this chunk must finish: x_S on [r0, r1) and, for the coarse rows it owns (fine row 2jc inside
     // the chunk AND inside the slab), r on [2jc-1, 2jc+1], i.e. x_S two rows earlier and one row later.
+    // (The pointwise first sweep needs no rows around the one it finishes: x_S row i depends on f rows i - SD .. i + SD.)
     const int lead = RESID ? 2 : 0;
-    int j_start_ = min(r0, max(r0, 0) - lead) - S;
+    int j_start_ = min(r0, max(r0, 0) - lead) - SD;
     if (PIN) j_start_ -= (j_start_ & 1);  // even: the row parity of the prolongation is static in the unrolled body
     const int j_start = j_start_;
-    const int j_end = max(r1 - 1, min(r1, g.ny) - 1 + (RESID ? 1 : 0)) + S;  // inclusive
+    const int j_end = max(r1 - 1, min(r1, g.ny) - 1 + (RESID ? 1 : 0)) + SD;  // inclusive
 
     SweepStage<C> st[S];
     ResidualStage<C> rs;
@@ -714,18 +751,21 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
                 for (int k = 0; k < C; ++k)
                     if (rowp && cprol[k]) cur.v[k] = add_correction(cur.v[k], corr[k], u & 1, k & 1);
             }
-            // sweeps: stage k consumes x_k row jj-k and finishes x_{k+1} row jj-k-1
+            // PW: cur = x_1 row jj, formed from f row jj alone
+            if (PW)
+                cur = sweep_row_from_zero<C, WEIGHTED>(feed.f_row(0), coef, jj + g.yoff > 0 && jj + g.yoff < g.n - 1, cin);
+            // sweeps: stage k consumes row jj-k of its input and finishes row jj-k-1 of its output
 #pragma unroll
-            for (int k = 0; k < S; ++k) {
+            for (int k = 0; k < SD; ++k) {
                 const int out_row = jj - k - 1 + g.yoff;  // global row
                 cur = st[k].template step<WEIGHTED>(u & 1, cur, feed.f_row(k), coef, out_row > 0 && out_row < g.n - 1, cin);
             }
-            // cur = x_S row jj - S
-            const int xrow = jj - S;
-            if (owner && xrow >= r0 && xrow < r1) store_row<C>(xo + (ptrdiff_t)xrow * g.pitch + col, cur);
+            // cur = x_S row jj - SD
+            const int xrow = jj - SD;
+            if (!NO_XB && owner && xrow >= r0 && xrow < r1) store_row<C>(xo + (ptrdiff_t)xrow * g.pitch + col, cur);
             if (RESID) {
-                Row<C> r = rs.step(u & 1, cur, feed.f_row(S + 1), inv_h2);  // r of row jj - S - 1
-                const int rrow = jj - S - 1;
+                Row<C> r = rs.step(u & 1, cur, feed.f_row(SD + 1), inv_h2);  // r of row jj - SD - 1
+                const int rrow = jj - SD - 1;
                 double left = __shfl_up_sync(0xffffffffu, r.v[C - 1], 1);
                 if (rrow & 1) {
                     // north row 2jc+1 of coarse row jc: finish the stencil
@@ -771,14 +811,18 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
 // ---------------------------------------------------------------------------------------------------
 // Pass B.  x = S^nu2(xb + P e) ; NORM adds sum over the interior of (f - A x)^2 (one partial per warp).
 // PROLONG = false makes it a plain smoothing (+norm) pass.
+// REBUILD = nu1 > 0 (one GPU, first visit, Pass A ran with NO_XB): xb = S^nu1(0; f) is not read but rebuilt from f ahead of
+// the prolongation -- a pointwise sweep (sweep_row_from_zero) and nu1 - 1 sweep stages -- so the pass reads f and e and
+// writes x: 18 B/point, and Pass A drops its 8 B/point xb store.
 // ---------------------------------------------------------------------------------------------------
-template <int C, int PF, int MINB, bool SM, int S, bool PROLONG, bool NORM, bool WEIGHTED>
+template <int C, int PF, int MINB, bool SM, int S, bool PROLONG, bool NORM, bool WEIGHTED, int REBUILD = 0>
 __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
     k_up(const double *__restrict__ xb, double *__restrict__ xo, const double *__restrict__ f,
          const double *__restrict__ e, StripGeom g, int pitch_c, int lo, JacobiCoef coef, double inv_h2,
          double *__restrict__ partials, const int *__restrict__ done)
 {
-    using Feed = typename FeedSelect<C, PF, S, true, SM>::type;
+    constexpr int D1 = REBUILD > 0 ? REBUILD - 1 : 0;  // rebuild sweep stages with a row of delay
+    using Feed = typename FeedSelect<C, PF, S + D1, REBUILD == 0, SM>::type;
     pdl_wait();
     const bool pdl_early = gridDim.x <= 296u;  // at most two CTAs per SM: a latency-bound level (pmg_internal.h)
     if (pdl_early) pdl_trigger();
@@ -794,11 +838,20 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
     bool owner, cin[C];
     strip_setup<C>(g, wid, lane, col, r0, r1, owner, cin);
 
-    // r0 is even; start on an even row so that row parity is static inside the unrolled body
-    int j_start = r0 - S - (NORM ? 1 : 0);
+    // r0 is even; start on an even row so that row parity is static inside the unrolled body.  jj (below) is the row of xb
+    // that enters the prolongation; with REBUILD the feed delivers f row jj + D1 and xb row jj leaves the rebuild stages.
+    // xb row i is exact once the feed started at row i - D1 or earlier, or at a row <= 1: rows <= 0 are Dirichlet or padding
+    // rows, zero in every sweep, so the zeroed stage state is then exact.  (Hence the clamp, which keeps the feed inside
+    // the PADY padding rows: the rebuild runs on whole levels only.)
+    int j_start = r0 - S - (NORM ? 1 : 0) - 2 * D1;
+    if (REBUILD > 0) j_start = max(j_start, -PADY - D1);
     j_start -= (j_start & 1);
+    if (REBUILD > 0 && j_start + D1 < -PADY) j_start += 2;  // a clamped start: the feed's first row is still <= 1
     const int j_end = r1 - 1 + S + (NORM ? 1 : 0);
 
+    SweepStage<C> pre[D1 > 0 ? D1 : 1];
+#pragma unroll
+    for (int k = 0; k < D1; ++k) pre[k].init();
     SweepStage<C> st[S];
     ResidualStage<C> rs;
 #pragma unroll
@@ -811,7 +864,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
     for (int k = 0; k < C; ++k) cprol[k] = (col + k >= lo) && (col + k <= g.n - 2);
 
     Feed feed;
-    feed.init(xb, f, g.pitch, col, j_start, g.ny + PADY - 1, lane, threadIdx.x >> 5, HaloPeers{}, g.ny);
+    feed.init(xb, f, g.pitch, col, j_start + D1, g.ny + PADY - 1, lane, threadIdx.x >> 5, HaloPeers{}, g.ny);
 
     // coarse rows: ec = row jc, en = row jc+1, eb = prefetch of row jc+2 (raw, before the shuffle)
     const int cc = col >> 1;
@@ -830,7 +883,15 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
 #pragma unroll
         for (int u = 0; u < Feed::UNROLL; ++u) {
             const int jj = j + u;  // u even: fine row 2jc, u odd: fine row 2jc+1
-            Row<C> cur = feed.begin(u, jj);
+            Row<C> cur = feed.begin(u, jj + D1);
+            if (REBUILD > 0) {  // cur = xb row jj: the pointwise first sweep on f row jj + D1, then D1 sweep stages
+                cur = sweep_row_from_zero<C, WEIGHTED>(feed.f_row(0), coef, jj + D1 + g.yoff > 0 && jj + D1 + g.yoff < g.n - 1, cin);
+#pragma unroll
+                for (int k = 0; k < D1; ++k) {
+                    const int out_row = jj + D1 - k - 1 + g.yoff;
+                    cur = pre[k].template step<WEIGHTED>(u & 1, cur, feed.f_row(k), coef, out_row > 0 && out_row < g.n - 1, cin);
+                }
+            }
             if (PROLONG) {
                 const bool rowp = (jj + g.yoff >= lo) && (jj + g.yoff <= g.n - 2);
                 double corr[C];  // the coarse values each point interpolates, summed but not yet weighted
@@ -860,12 +921,12 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
 #pragma unroll
             for (int k = 0; k < S; ++k) {
                 const int out_row = jj - k - 1 + g.yoff;
-                cur = st[k].template step<WEIGHTED>(u & 1, cur, feed.f_row(k), coef, out_row > 0 && out_row < g.n - 1, cin);
+                cur = st[k].template step<WEIGHTED>(u & 1, cur, feed.f_row(D1 + k), coef, out_row > 0 && out_row < g.n - 1, cin);
             }
             const int xrow = jj - S;
             if (owner && xrow >= r0 && xrow < r1) store_row<C>(xo + (ptrdiff_t)xrow * g.pitch + col, cur);
             if (NORM) {
-                Row<C> r = rs.step(u & 1, cur, feed.f_row(S + 1), inv_h2);
+                Row<C> r = rs.step(u & 1, cur, feed.f_row(D1 + S + 1), inv_h2);
                 const int rrow = jj - S - 1;
                 if (owner && rrow >= r0 && rrow < r1 && rrow >= 0 && rrow < g.ny && rrow + g.yoff > 0 &&
                     rrow + g.yoff < g.n - 1) {
@@ -1262,7 +1323,7 @@ inline int current_device()
     } while (0)
 
 template <int C, int PF, int MINB, bool SM, int S, bool WEIGHTED>
-void down_launch_w(const FusedLevel &lv, double *cf, int pitch_c, bool x_is_zero, bool resid, const StripGeom &g,
+void down_launch_w(const FusedLevel &lv, double *cf, int pitch_c, bool x_is_zero, bool resid, bool store_xb, const StripGeom &g,
                    int nc, const JacobiCoef &c, double inv, dim3 grid, dim3 block, const int *done, cudaStream_t st)
 {
     // the halo-prologue flavour exists for the headline sweep count on the shared-memory feed only
@@ -1276,6 +1337,11 @@ void down_launch_w(const FusedLevel &lv, double *cf, int pitch_c, bool x_is_zero
     } else if (resid && prologue) {
         auto k = k_down<C, PF, MINB, SM, S, false, true, WEIGHTED, CAN_PROLOGUE>;
         int sm = WARPS_PER_CTA * FeedSelect<C, PF, S, true, SM>::type::SMEM_PER_WARP;
+        PMG_SMEM_ONCE(k, sm);
+        PMG_LAUNCH(k, grid, block, sm, st, lv.x, lv.xb, lv.f, cf, g, pitch_c, nc, c, inv, done, lv.hp, (const double *)nullptr, 0, 0);
+    } else if (resid && x_is_zero && !store_xb) {
+        auto k = k_down<C, PF, MINB, SM, S, true, true, WEIGHTED, false, false, true>;
+        int sm = WARPS_PER_CTA * FeedSelect<C, PF, S, false, SM>::type::SMEM_PER_WARP;
         PMG_SMEM_ONCE(k, sm);
         PMG_LAUNCH(k, grid, block, sm, st, lv.x, lv.xb, lv.f, cf, g, pitch_c, nc, c, inv, done, lv.hp, (const double *)nullptr, 0, 0);
     } else if (resid && x_is_zero) {
@@ -1297,7 +1363,7 @@ void down_launch_w(const FusedLevel &lv, double *cf, int pitch_c, bool x_is_zero
 }
 
 template <int C, int PF, int MINB, bool SM, int S>
-void down_launch(const FusedLevel &lv, double *cf, int pitch_c, double omega, bool x_is_zero, bool resid,
+void down_launch(const FusedLevel &lv, double *cf, int pitch_c, double omega, bool x_is_zero, bool resid, bool store_xb,
                  const int *done, cudaStream_t st)
 {
     StripGeom g = make_geom(lv, S + (resid ? 2 : 0), VariantDesc{C, PF, MINB, SM}, lv.ext_lo, lv.ext_hi);
@@ -1306,9 +1372,9 @@ void down_launch(const FusedLevel &lv, double *cf, int pitch_c, double omega, bo
     int nc = (lv.n - 1) / 2 + 1;
     dim3 grid(grid_for(g)), block(32 * WARPS_PER_CTA);
     if (c.weighted) {
-        down_launch_w<C, PF, MINB, SM, S, true>(lv, cf, pitch_c, x_is_zero, resid, g, nc, c, inv, grid, block, done, st);
+        down_launch_w<C, PF, MINB, SM, S, true>(lv, cf, pitch_c, x_is_zero, resid, store_xb, g, nc, c, inv, grid, block, done, st);
     } else {
-        down_launch_w<C, PF, MINB, SM, S, false>(lv, cf, pitch_c, x_is_zero, resid, g, nc, c, inv, grid, block, done, st);
+        down_launch_w<C, PF, MINB, SM, S, false>(lv, cf, pitch_c, x_is_zero, resid, store_xb, g, nc, c, inv, grid, block, done, st);
     }
     count_launch();
 }
@@ -1329,12 +1395,12 @@ void down_prolong_launch_w(const FusedLevel &lv, const double *e_in, int pitch_e
                HaloPeers{}, e_in, pitch_e, lo);
 }
 
-template <int C, int PF, int MINB, bool SM, int S, bool PROLONG, bool NORM, bool WEIGHTED>
+template <int C, int PF, int MINB, bool SM, int S, bool PROLONG, bool NORM, bool WEIGHTED, int REBUILD = 0>
 void up_launch_k(const FusedLevel &lv, const double *e, int pitch_c, const StripGeom &g, int lo,
                  const JacobiCoef &c, double inv, double *d_partials, const int *done, cudaStream_t st)
 {
-    auto k = k_up<C, PF, MINB, SM, S, PROLONG, NORM, WEIGHTED>;
-    int sm = WARPS_PER_CTA * FeedSelect<C, PF, S, true, SM>::type::SMEM_PER_WARP;
+    auto k = k_up<C, PF, MINB, SM, S, PROLONG, NORM, WEIGHTED, REBUILD>;
+    int sm = WARPS_PER_CTA * FeedSelect<C, PF, S + (REBUILD > 0 ? REBUILD - 1 : 0), REBUILD == 0, SM>::type::SMEM_PER_WARP;
     PMG_SMEM_ONCE(k, sm);
     PMG_LAUNCH(k, dim3(grid_for(g)), dim3(32 * WARPS_PER_CTA), sm, st, lv.xb, lv.x, lv.f, e, g, pitch_c, lo, c, inv, d_partials, done);
 }
@@ -1369,6 +1435,34 @@ void up_launch(const FusedLevel &lv, const double *e, int pitch_c, double omega,
     }
     count_launch();
     if (n_partials) *n_partials = norm ? g.n_strips * g.n_chunks : 0;
+}
+
+// Pass B of a first visit that rebuilds xb = S^nu1(0; f) (k_up with REBUILD = nu1): prolongation, no norm, whole level.
+// One shape per sweep count: the Pass B variant the solve uses by default.
+template <int C, int PF, int MINB, bool SM, int S, int NU1>
+void up_rebuild_launch(const FusedLevel &lv, const double *e, int pitch_c, double omega, int lo, const int *done, cudaStream_t st)
+{
+    StripGeom g = make_geom(lv, (NU1 - 1) + S + 1, VariantDesc{C, PF, MINB, SM}, lv.ext_lo, lv.ext_hi);
+    JacobiCoef c = jacobi_coef(lv.h, omega);
+    double inv = 1.0 / (lv.h * lv.h);
+    if (c.weighted)
+        up_launch_k<C, PF, MINB, SM, S, true, false, true, NU1>(lv, e, pitch_c, g, lo, c, inv, nullptr, done, st);
+    else
+        up_launch_k<C, PF, MINB, SM, S, true, false, false, NU1>(lv, e, pitch_c, g, lo, c, inv, nullptr, done, st);
+    count_launch();
+}
+
+template <int C, int PF, int MINB, bool SM, int S>
+void up_rebuild_dispatch(const FusedLevel &lv, const double *e, int pitch_c, double omega, int lo, int nu1, const int *done,
+                         cudaStream_t st)
+{
+    switch (nu1) {
+        case 1: up_rebuild_launch<C, PF, MINB, SM, S, 1>(lv, e, pitch_c, omega, lo, done, st); break;
+        case 2: up_rebuild_launch<C, PF, MINB, SM, S, 2>(lv, e, pitch_c, omega, lo, done, st); break;
+        case 3: up_rebuild_launch<C, PF, MINB, SM, S, 3>(lv, e, pitch_c, omega, lo, done, st); break;
+        case 4: up_rebuild_launch<C, PF, MINB, SM, S, 4>(lv, e, pitch_c, omega, lo, done, st); break;
+        default: break;
+    }
 }
 
 // geometry of the cross-cycle pass: 4 sweeps + residual + restriction eat 6 columns per side
@@ -1492,6 +1586,33 @@ void fused_set_variant(int v)
 }
 int fused_get_variant() { return g_variant_down | (g_variant_up << 8); }
 void fused_set_min_chunk_rows(int r) { g_min_chunk_rows = (r >= 2) ? (r + (r & 1)) : 2; }
+
+int g_rebuild_xb = -2;  // -2: not yet read from PMG_REBUILD_XB
+void fused_set_rebuild_xb(int mode) { g_rebuild_xb = (mode == 0 || mode == 1) ? mode : -1; }
+static size_t l2_bytes()
+{
+#ifdef PMG_HOST_EMULATION
+    return (size_t)126 << 20;
+#else
+    int dev = 0, v = 0;
+    cudaGetDevice(&dev);
+    static int cached[64] = {};
+    int &c = cached[dev & 63];
+    if (c == 0) c = (cudaDeviceGetAttribute(&v, cudaDevAttrL2CacheSize, dev) == cudaSuccess && v > 0) ? v : -1;
+    return c > 0 ? (size_t)c : 0;
+#endif
+}
+bool fused_rebuild_xb(const FusedLevel &lv, int nu1)
+{
+    if (g_rebuild_xb == -2) {
+        const char *e = getenv("PMG_REBUILD_XB");
+        g_rebuild_xb = (e && (e[0] == '0' || e[0] == '1')) ? e[0] - '0' : -1;
+    }
+    if (lv.ny != 0 || !fused_supported(nu1) || g_rebuild_xb == 0) return false;
+    if (g_rebuild_xb == 1) return true;
+    const size_t l2 = l2_bytes();
+    return l2 > 0 && 3 * level_elems(lv.n) * sizeof(double) > l2;
+}
 void fused_set_deep_prefetch_below(int n) { g_deep_prefetch_below = n; }
 void fused_set_halo_prologue(int on) { g_halo_prologue = on ? 1 : 0; }
 void fused_set_wait_timeout_ns(unsigned long long ns)
@@ -1531,18 +1652,19 @@ int fused_max_partials(int n)
     }
 
 void launch_fused_down(const FusedLevel &lv, double *coarse_f, int pitch_c, int nu1, double omega,
-                       bool x_is_zero, cudaStream_t st, const int *done)
+                       bool x_is_zero, cudaStream_t st, const int *done, bool store_xb)
 {
     bool resid = coarse_f != nullptr;
-    if (!fused_supported(nu1)) {  // callers check fused_supported(); never skip a pass silently
-        g_fused_bad_nu = nu1;
+    // the xb store is skipped only where Pass B can rebuild xb: a first visit of a whole level
+    if (!fused_supported(nu1) || (!store_xb && !(x_is_zero && resid && lv.ny == 0))) {  // never skip a pass silently
+        g_fused_bad_nu = fused_supported(nu1) ? -1 : nu1;
         return;
     }
     switch (nu1) {
-        case 1: down_launch<2, 3, 4, true, 1>(lv, coarse_f, pitch_c, omega, x_is_zero, resid, done, st); break;
-        case 2: PMG_DISPATCH_S2(lv.n <= deep_prefetch_below() ? 4 : ((x_is_zero && resid) ? g_variant_down_zero : g_variant_down), down_launch, lv, coarse_f, pitch_c, omega, x_is_zero, resid, done, st); break;
-        case 3: down_launch<2, 3, 4, true, 3>(lv, coarse_f, pitch_c, omega, x_is_zero, resid, done, st); break;
-        case 4: down_launch<2, 2, 4, true, 4>(lv, coarse_f, pitch_c, omega, x_is_zero, resid, done, st); break;
+        case 1: down_launch<2, 3, 4, true, 1>(lv, coarse_f, pitch_c, omega, x_is_zero, resid, store_xb, done, st); break;
+        case 2: PMG_DISPATCH_S2(lv.n <= deep_prefetch_below() ? 4 : ((x_is_zero && resid) ? g_variant_down_zero : g_variant_down), down_launch, lv, coarse_f, pitch_c, omega, x_is_zero, resid, store_xb, done, st); break;
+        case 3: down_launch<2, 3, 4, true, 3>(lv, coarse_f, pitch_c, omega, x_is_zero, resid, store_xb, done, st); break;
+        case 4: down_launch<2, 2, 4, true, 4>(lv, coarse_f, pitch_c, omega, x_is_zero, resid, store_xb, done, st); break;
         default: break;
     }
 }
@@ -1563,13 +1685,28 @@ void launch_fused_down_prolong(const FusedLevel &lv, const double *e_in, int pit
 }
 
 void launch_fused_up(const FusedLevel &lv, const double *coarse_x, int pitch_c, int nu2, double omega,
-                     int prolong_mode, double *d_partials, int *n_partials, cudaStream_t st, const int *done)
+                     int prolong_mode, double *d_partials, int *n_partials, cudaStream_t st, const int *done, int rebuild_nu1)
 {
     bool norm = d_partials != nullptr;
     int lo = prolong_mode == PMG_PROLONG_FULL ? 1 : 2;
     if (!fused_supported(nu2)) {
         g_fused_bad_nu = nu2;
         if (n_partials) *n_partials = 0;
+        return;
+    }
+    if (rebuild_nu1 != 0) {  // xb rebuilt from f: whole level, with a prolongation, without the norm
+        if (n_partials) *n_partials = 0;
+        if (!fused_supported(rebuild_nu1) || norm || coarse_x == nullptr || lv.ny != 0) {
+            g_fused_bad_nu = fused_supported(rebuild_nu1) ? -1 : rebuild_nu1;
+            return;
+        }
+        switch (nu2) {
+            case 1: up_rebuild_dispatch<2, 3, 4, true, 1>(lv, coarse_x, pitch_c, omega, lo, rebuild_nu1, done, st); break;
+            case 2: up_rebuild_dispatch<2, 3, 5, true, 2>(lv, coarse_x, pitch_c, omega, lo, rebuild_nu1, done, st); break;
+            case 3: up_rebuild_dispatch<2, 3, 4, true, 3>(lv, coarse_x, pitch_c, omega, lo, rebuild_nu1, done, st); break;
+            case 4: up_rebuild_dispatch<2, 2, 4, true, 4>(lv, coarse_x, pitch_c, omega, lo, rebuild_nu1, done, st); break;
+            default: break;
+        }
         return;
     }
     switch (nu2) {

@@ -319,16 +319,25 @@ bool fused_down_prolong_supported(int nu1);
 void launch_fused_down_prolong(const FusedLevel &lv, const double *e_in, int pitch_e, double *coarse_f, int pitch_c, double omega,
                                int prolong_mode, cudaStream_t st, const int *done = nullptr);
 // a launcher called with an unsupported sweep count launches nothing and records the count; returns and clears it
-// (0 = none): the cycle drivers turn it into PMG_ERR_UNSUPPORTED instead of a silently skipped pass
+// (0 = none; -1 = a store_xb / rebuild_nu1 request outside a first visit of a whole level): the cycle drivers turn it
+// into PMG_ERR_UNSUPPORTED instead of a silently skipped pass
 int fused_take_bad_nu();
 // `done` (nullable): device flag; when set the kernel returns at once (device-side convergence control)
+// store_xb = false (x_is_zero, coarse_f, whole level only): xb is not written; Pass B must then rebuild it (rebuild_nu1)
 void launch_fused_down(const FusedLevel &lv, double *coarse_f, int pitch_c, int nu1, double omega,
-                       bool x_is_zero, cudaStream_t st, const int *done = nullptr);
+                       bool x_is_zero, cudaStream_t st, const int *done = nullptr, bool store_xb = true);
 // Pass B (up): x = S^nu2(xb + P coarse_x); optionally sum (f - A x)^2 over the interior into partials
 // (count returned through *n_partials; reduce with launch_final_sum)
+// rebuild_nu1 > 0 (whole level, coarse_x, no norm): xb is not read but rebuilt as S^nu1(0; f) -- after a Pass A with
+// x_is_zero and store_xb = false
 void launch_fused_up(const FusedLevel &lv, const double *coarse_x, int pitch_c, int nu2, double omega,
                      int prolong_mode, double *d_partials, int *n_partials, cudaStream_t st,
-                     const int *done = nullptr);
+                     const int *done = nullptr, int rebuild_nu1 = 0);
+// Whether a first visit (x == 0) of this level skips the xb store and rebuilds xb in Pass B: whole levels whose three
+// arrays (x, xb, f) exceed the L2 cache.  Below that the xb store and read stay in L2 and cost less than the extra sweep.
+bool fused_rebuild_xb(const FusedLevel &lv, int nu1);
+// -1: by size (default; PMG_REBUILD_XB=0/1 in the environment overrides it), 0: never, 1: on every whole level
+void fused_set_rebuild_xb(int mode);
 int fused_max_partials(int n);
 // Cross-cycle pass (level 0 of a V-cycle solve, one GPU): Pass B of cycle k and Pass A of cycle k+1 in one sweep over
 // HBM -- reads lv.xb (xb_k), coarse_x (e_k), lv.f; writes lv.x (x_k), xb_out (xb_{k+1}, NOT lv.xb), coarse_f and the partial

@@ -390,18 +390,20 @@ static pmg_status cycle_fused(pmg_solver *s, int l, bool w_form, bool x_is_zero,
         return PMG_OK;
     }
     Level &K = s->lv[l + 1];
+    // a large first visit does not store xb: Pass B rebuilds it from f (which no coarser visit changes)
+    const bool rebuild = prolong_in == nullptr && x_is_zero && !want_norm && fused_rebuild_xb(fused_view(L), c.nu1);
     if (prolong_in != nullptr)
         launch_fused_down_prolong(fused_view(L), prolong_in->x, prolong_in->pitch, K.f, K.pitch, c.omega, c.prolong_mode,
                                   s->stream, done);
     else
-        launch_fused_down(fused_view(L), K.f, K.pitch, c.nu1, c.omega, x_is_zero, s->stream, done);
+        launch_fused_down(fused_view(L), K.f, K.pitch, c.nu1, c.omega, x_is_zero, s->stream, done, !rebuild);
     int reps = w_form ? c.gamma : 1;
     for (int k = 0; k < reps; ++k) {
         pmg_status rc = cycle_fused(s, l + 1, w_form, k == 0, false, nullptr, done);
         if (rc != PMG_OK) return rc;
     }
     launch_fused_up(fused_view(L), K.x, K.pitch, c.nu2, c.omega, c.prolong_mode,
-                    want_norm ? s->d_partials : nullptr, n_partials, s->stream, done);
+                    want_norm ? s->d_partials : nullptr, n_partials, s->stream, done, rebuild ? c.nu1 : 0);
     return PMG_OK;
 }
 
@@ -2331,6 +2333,9 @@ int pmg_cluster_top(const pmg_solver *s) { return s ? s->cluster_top : 0; }
 int pmg_fused_num_variants(void) { return fused_num_variants(); }
 void pmg_fused_set_variant(int v) { fused_set_variant(v); }
 void pmg_fused_set_min_chunk_rows(int r) { fused_set_min_chunk_rows(r); }
+/* first visits of whole levels: skip the xb store and rebuild xb in Pass B -- -1 by size (default), 0 never, 1 always;
+ * read when a cycle is recorded, so set it before the solver's first cycle */
+void pmg_fused_set_rebuild_xb(int mode) { fused_set_rebuild_xb(mode); }
 void pmg_fused_set_deep_prefetch_below(int n) { fused_set_deep_prefetch_below(n); }
 void pmg_fused_set_halo_prologue(int on) { fused_set_halo_prologue(on); }
 
@@ -2431,7 +2436,8 @@ pmg_status pmg_smooth(pmg_solver *s, int sweeps, int block)
 
 /* Times one fused pass of level `level` in isolation: which = 0 Pass A (sweeps+residual+restriction),
  * 1 Pass B with the residual norm, 2 Pass B without, 3 Pass A with x == 0 (coarse-level form), 4 the cross-cycle pass
- * (Pass B of one cycle + Pass A of the next; level 0, one GPU, x_k not written as in pmg_solve).  `reps`
+ * (Pass B of one cycle + Pass A of the next; level 0, one GPU, x_k not written as in pmg_solve), 5 Pass A with x == 0
+ * without the xb store, 6 Pass B rebuilding xb from f (the pair a large first visit runs instead of 3 and 2).  `reps`
  * launches between two CUDA events on the solver stream; *ms_avg = average per launch.  Clobbers the
  * iterate (benchmark use only). */
 pmg_status pmg_bench_pass(pmg_solver *s, int which, int level, int reps, double *ms_avg)
@@ -2455,11 +2461,11 @@ pmg_status pmg_bench_pass(pmg_solver *s, int which, int level, int reps, double 
             v.x = nullptr;
             use_rhs_tables(s, v);  // the flavour pmg_solve runs
             launch_fused_cross(v, s->xc, K.x, K.f, K.pitch, c.omega, c.prolong_mode, s->d_partials, &np, s->stream);
-        } else if (which == 0 || which == 3)
-            launch_fused_down(fused_view(L), K.f, K.pitch, c.nu1, c.omega, which == 3, s->stream);
+        } else if (which == 0 || which == 3 || which == 5)
+            launch_fused_down(fused_view(L), K.f, K.pitch, c.nu1, c.omega, which != 0, s->stream, nullptr, which != 5);
         else
             launch_fused_up(fused_view(L), K.x, K.pitch, c.nu2, c.omega, c.prolong_mode,
-                            which == 1 ? s->d_partials : nullptr, &np, s->stream);
+                            which == 1 ? s->d_partials : nullptr, &np, s->stream, nullptr, which == 6 ? c.nu1 : 0);
     };
     one();  // warm-up
     PMG_CUDA(cudaEventRecord(s->ev0, s->stream));
@@ -2469,6 +2475,7 @@ pmg_status pmg_bench_pass(pmg_solver *s, int which, int level, int reps, double 
     PMG_CUDA(cudaGetLastError());
     float ms = 0.f;
     PMG_CUDA(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
+    if (fused_take_bad_nu()) return fail(PMG_ERR_UNSUPPORTED, "this pass form needs a whole level (one GPU)");
     *ms_avg = ms / reps;
     return PMG_OK;
 }
