@@ -1230,6 +1230,9 @@ int deep_prefetch_below()
 int g_variant_down = 0, g_variant_down_zero = 3, g_variant_up = 1, g_variant_up_norm = 3;
 
 int g_fused_bad_nu = 0;  // last sweep count a launcher was asked for and could not serve (fused_take_bad_nu)
+// a launcher refuses a pass: record the sweep count it has no kernel for, or -1 for a form the level cannot take -- and
+// for a count of 0, which would otherwise read as "nothing refused"
+void refuse(int nu) { g_fused_bad_nu = (nu != 0 && !fused_supported(nu)) ? nu : -1; }
 
 int g_min_chunk_rows = 4;  // even; the pipeline warm-up (4..8 rows) is paid once per chunk
 
@@ -1505,6 +1508,14 @@ int fused_take_bad_nu()
 constexpr int PMG_CROSS_SHAPE_DEFAULT = 2;
 int g_cross_minb = PMG_CROSS_SHAPE_DEFAULT;
 bool fused_cross_supported(int nu1, int nu2) { return nu1 == 2 && nu2 == 2; }
+// grid of the cross-cycle pass in shape m (launch_fused_cross); *minb = CTAs per SM of that shape
+static StripGeom cross_geom(const FusedLevel &lv, int m, int *minb)
+{
+    const bool wide = (m == 2 || m == 7) && (lv.n - 1) % 4 == 0;
+    VariantDesc v{wide ? 4 : 2, 2, wide ? 2 : (m == 4 || m == 5 || m == 6 ? m : 3), 1};
+    *minb = v.minb;
+    return make_geom(lv, 6, v, 0, 0, wide ? 8 : 6);
+}
 // Fraction of the resident warp slots the cross-cycle pass fills on an n-column level of `rows` rows.  The grid is one
 // resident wave of (strips x chunks) warps with chunks = floor(slots / strips): at n = 32769 the 631 strips of 52 columns
 // leave 3 chunks = 80 % of the slots (the two-pass kernels' 586 strips of 56 columns give 4 chunks = 99 %), and the pass
@@ -1516,10 +1527,9 @@ double fused_cross_utilisation(int n, int rows)
     lv.n = n;
     lv.ny = rows;
     lv.pitch = level_pitch(n);
-    const bool wide = g_cross_minb == 2 || g_cross_minb == 7;
-    VariantDesc v{wide ? 4 : 2, 2, wide ? 2 : g_cross_minb, 1};
-    StripGeom g = make_geom(lv, 6, v, 0, 0, wide ? 8 : 6);
-    return (double)(g.n_strips * g.n_chunks) / (double)(num_sms() * v.minb * WARPS_PER_CTA);
+    int minb = 0;
+    StripGeom g = cross_geom(lv, g_cross_minb, &minb);
+    return (double)(g.n_strips * g.n_chunks) / (double)(num_sms() * minb * WARPS_PER_CTA);
 }
 void fused_set_cross_minb(int m) { g_cross_minb = (m >= 2 && m <= 7) ? m : PMG_CROSS_SHAPE_DEFAULT; }
 void launch_fused_cross(const FusedLevel &lv, double *xb_out, const double *coarse_x, double *coarse_f, int pitch_c, double omega,
@@ -1624,6 +1634,23 @@ void fused_set_wait_timeout_ns(unsigned long long ns)
 #endif
 }
 int fused_halo_prologue() { return g_halo_prologue; }
+FusedTuning fused_get_tuning()
+{
+    return FusedTuning{g_variant_down, g_variant_down_zero, g_variant_up, g_variant_up_norm, g_cross_minb,
+                       g_min_chunk_rows, g_deep_prefetch_below, g_rebuild_xb, g_halo_prologue};
+}
+void fused_set_tuning(const FusedTuning &t)
+{
+    g_variant_down = t.variant_down;
+    g_variant_down_zero = t.variant_down_zero;
+    g_variant_up = t.variant_up;
+    g_variant_up_norm = t.variant_up_norm;
+    g_cross_minb = t.cross_minb;
+    g_min_chunk_rows = t.min_chunk_rows;
+    g_deep_prefetch_below = t.deep_prefetch_below;
+    g_rebuild_xb = t.rebuild_xb;
+    g_halo_prologue = t.halo_prologue;
+}
 
 int fused_max_partials(int n)
 {
@@ -1637,6 +1664,12 @@ int fused_max_partials(int n)
         g = make_geom(lv, 4, VARIANTS[v], 8, 8);
         if (g.n_strips * g.n_chunks > c) c = g.n_strips * g.n_chunks;
         if (c > best) best = c;
+    }
+    // the cross-cycle pass: strips of 52 columns (halo 6) give more warps than any two-pass strip width
+    for (int m = 2; m <= 7; ++m) {
+        int minb = 0;
+        StripGeom g = cross_geom(lv, m, &minb);
+        if (g.n_strips * g.n_chunks > best) best = g.n_strips * g.n_chunks;
     }
     return best + 64;
 }
@@ -1657,7 +1690,7 @@ void launch_fused_down(const FusedLevel &lv, double *coarse_f, int pitch_c, int 
     bool resid = coarse_f != nullptr;
     // the xb store is skipped only where Pass B can rebuild xb: a first visit of a whole level
     if (!fused_supported(nu1) || (!store_xb && !(x_is_zero && resid && lv.ny == 0))) {  // never skip a pass silently
-        g_fused_bad_nu = fused_supported(nu1) ? -1 : nu1;
+        refuse(nu1);
         return;
     }
     switch (nu1) {
@@ -1690,14 +1723,14 @@ void launch_fused_up(const FusedLevel &lv, const double *coarse_x, int pitch_c, 
     bool norm = d_partials != nullptr;
     int lo = prolong_mode == PMG_PROLONG_FULL ? 1 : 2;
     if (!fused_supported(nu2)) {
-        g_fused_bad_nu = nu2;
+        refuse(nu2);
         if (n_partials) *n_partials = 0;
         return;
     }
     if (rebuild_nu1 != 0) {  // xb rebuilt from f: whole level, with a prolongation, without the norm
         if (n_partials) *n_partials = 0;
         if (!fused_supported(rebuild_nu1) || norm || coarse_x == nullptr || lv.ny != 0) {
-            g_fused_bad_nu = fused_supported(rebuild_nu1) ? -1 : rebuild_nu1;
+            refuse(rebuild_nu1);
             return;
         }
         switch (nu2) {

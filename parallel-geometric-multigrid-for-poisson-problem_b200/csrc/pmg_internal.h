@@ -319,8 +319,8 @@ bool fused_down_prolong_supported(int nu1);
 void launch_fused_down_prolong(const FusedLevel &lv, const double *e_in, int pitch_e, double *coarse_f, int pitch_c, double omega,
                                int prolong_mode, cudaStream_t st, const int *done = nullptr);
 // a launcher called with an unsupported sweep count launches nothing and records the count; returns and clears it
-// (0 = none; -1 = a store_xb / rebuild_nu1 request outside a first visit of a whole level): the cycle drivers turn it
-// into PMG_ERR_UNSUPPORTED instead of a silently skipped pass
+// (0 = none; -1 = a store_xb / rebuild_nu1 request outside a first visit of a whole level, or a sweep count of 0): the
+// cycle drivers turn it into PMG_ERR_UNSUPPORTED instead of a silently skipped pass
 int fused_take_bad_nu();
 // `done` (nullable): device flag; when set the kernel returns at once (device-side convergence control)
 // store_xb = false (x_is_zero, coarse_f, whole level only): xb is not written; Pass B must then rebuild it (rebuild_nu1)
@@ -364,6 +364,14 @@ void fused_set_deep_prefetch_below(int n);
 constexpr int PMG_HALO_PROLOGUE_DEFAULT = 1;
 void fused_set_halo_prologue(int on);
 int fused_halo_prologue();
+// every tuning switch of the fused passes above (variants, cross-pass shape, chunk rows, deep prefetch, xb rebuild, halo
+// prologue), read and written as a whole so that a caller can run one pass under other settings and put them back
+struct FusedTuning {
+    int variant_down, variant_down_zero, variant_up, variant_up_norm, cross_minb, min_chunk_rows, deep_prefetch_below,
+        rebuild_xb, halo_prologue;
+};
+FusedTuning fused_get_tuning();
+void fused_set_tuning(const FusedTuning &t);
 // limit of the peer-flag waits (wait_flag above), per translation unit that waits
 void fused_set_wait_timeout_ns(unsigned long long ns);
 void basic_set_wait_timeout_ns(unsigned long long ns);

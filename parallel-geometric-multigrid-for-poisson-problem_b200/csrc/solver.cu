@@ -2590,6 +2590,93 @@ void pmg_set_p2p_timeout_ms(double ms)
 
 int pmg_test_fused_max_partials(int n) { return fused_max_partials(n); }
 
+/* One fused pass over a WHOLE level (one GPU) on caller-built padded arrays, in each form the single-GPU solve launches,
+ * for the pass-by-pass comparison with the oracle (tests/test_gpu_fused_pass_matrix.py).  `form`:
+ *   0 Pass A smoothing only           xb = S^nu(x)
+ *   1 Pass A                          xb = S^nu(x),      coarse_f = R(f - A xb)
+ *   2 Pass A from x == 0              xb = S^nu(0),      coarse_f            (x not read)
+ *   3 Pass A from x == 0, no xb store                    coarse_f            (x not read, xb not written)
+ *   4 Pass A prolong-in (nu = 2)      xb = S^2(P coarse_x), coarse_f         (x not read)
+ *   5 Pass B                          x = S^nu(xb + P coarse_x) (coarse_x nullable: no prolongation), norm partials if
+ *                                     partials != null
+ *   6 Pass B rebuilding xb            x = S^nu(S^nu_pre(0) + P coarse_x)     (xb not read)
+ *   7 cross-cycle pass (nu = nu_pre = 2): x = S^2(xb + P coarse_x) (x nullable: not stored), its norm partials,
+ *                                     xb_out = S^2 x, coarse_f = R(f - A xb_out); f generated from rhs_fx / rhs_sy when
+ *                                     both are set (FusedLevel::rhs_fx)
+ * The pass runs under the given tuning (the setters' arguments: pmg_fused_set_variant, _cross_minb, _min_chunk_rows,
+ * _deep_prefetch_below); every tuning switch is put back afterwards.  A form no launcher serves is PMG_ERR_UNSUPPORTED. */
+typedef struct {
+    int form;
+    double *x, *xb;
+    const double *f;
+    int n, pitch;
+    double h;
+    const double *coarse_x;
+    double *coarse_f;
+    int pitch_c;
+    int nu, nu_pre;
+    double omega;
+    int prolong_mode;
+    double *partials;
+    int n_partials;  // out
+    double *xb_out;
+    const double *rhs_fx, *rhs_sy;
+    int variant, cross_shape, min_chunk_rows, deep_prefetch_below;
+} pmg_test_pass;
+
+pmg_status pmg_test_fused_pass(pmg_test_pass *t)
+{
+    if (!t || t->form < 0 || t->form > 7 || !is_pow2_plus_1(t->n) || (t->form == 6 && t->nu_pre == 0))
+        return fail(PMG_ERR_INVALID, "bad argument");
+    if ((t->form == 4 && !fused_down_prolong_supported(t->nu)) ||
+        (t->form == 7 && !fused_cross_supported(t->nu_pre, t->nu)))
+        return fail(PMG_ERR_UNSUPPORTED, "no kernel for this sweep count in this pass form");
+    pmg_status rc = require_device();
+    if (rc != PMG_OK) return rc;
+    FusedLevel v{};
+    v.x = t->x;
+    v.xb = t->xb;
+    v.f = t->f;
+    v.n = t->n;
+    v.pitch = t->pitch;
+    v.h = t->h;
+    const FusedTuning saved = fused_get_tuning();
+    fused_set_variant(t->variant);
+    fused_set_cross_minb(t->cross_shape);
+    fused_set_min_chunk_rows(t->min_chunk_rows);
+    fused_set_deep_prefetch_below(t->deep_prefetch_below);
+    t->n_partials = 0;
+    switch (t->form) {
+        case 0: launch_fused_down(v, nullptr, 0, t->nu, t->omega, false, nullptr); break;
+        case 1:
+        case 2:
+        case 3:
+            launch_fused_down(v, t->coarse_f, t->pitch_c, t->nu, t->omega, t->form != 1, nullptr, nullptr, t->form != 3);
+            break;
+        case 4:
+            launch_fused_down_prolong(v, t->coarse_x, t->pitch_c, t->coarse_f, t->pitch_c, t->omega, t->prolong_mode, nullptr);
+            break;
+        case 5:
+        case 6:
+            launch_fused_up(v, t->coarse_x, t->pitch_c, t->nu, t->omega, t->prolong_mode, t->partials, &t->n_partials,
+                            nullptr, nullptr, t->form == 6 ? t->nu_pre : 0);
+            break;
+        default:
+            v.rhs_fx = t->rhs_fx;
+            v.rhs_sy = t->rhs_sy;
+            launch_fused_cross(v, t->xb_out, t->coarse_x, t->coarse_f, t->pitch_c, t->omega, t->prolong_mode, t->partials,
+                               &t->n_partials, nullptr);
+            break;
+    }
+    fused_set_tuning(saved);
+    if (const int bad = fused_take_bad_nu())
+        return fail(PMG_ERR_UNSUPPORTED,
+                    "pass form " + std::to_string(t->form) + " launched nothing (" + std::to_string(bad) + ")");
+    PMG_CUDA(cudaDeviceSynchronize());
+    PMG_CUDA(cudaGetLastError());
+    return PMG_OK;
+}
+
 /* ---- operator level (dense reference layout, device pointers) ------------------------------------------ */
 // Scratch of the operator-level calls, one set PER DEVICE ordinal: reduction partials and the padded buffers of the
 // blocked smoother.  The calls are synchronous, and they hold g_scratch_mu from launch to completion, so concurrent
