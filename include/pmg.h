@@ -56,7 +56,8 @@ typedef enum pmg_cycle_kind {
      * reference's F-cycle regenerates the analytic RHS on every level, MultiGrid.hpp:162, and zeroes the ring).
      * The iterate's ring is kept, its interior restarted from 0: r0 = f - A x; f_1 = R r0, f_{l+1} = R f_l; coarsest
      * level: coarse_sweeps sweeps from 0; upwards e_l = P e_{l+1} and one V-cycle on (e_l, f_l); finest level
-     * x += P e_1 and one V-cycle on (x, f).  pmg_solve with this kind = one such pass, then V-cycles.  One GPU only.
+     * x += P e_1 and one V-cycle on (x, f).  pmg_solve with this kind = one such pass, then V-cycles.  One GPU, and
+     * row slabs too (n_ranks a power of two; otherwise PMG_ERR_UNSUPPORTED on every rank).
      * Specification: the CPU checker's orc_fmg_general, which the GPU result equals bit for bit. */
     PMG_CYCLE_FMG = 3
 } pmg_cycle_kind;
@@ -246,8 +247,9 @@ int pmg_device_count(void);
  *      torch.distributed).  With n_ranks > 1 the solver partitions every fine level into row slabs; pmg_set_rhs /
  *      pmg_set_guess / pmg_get_solution then move THIS RANK'S rows [y0, y1) (pmg_partition_rows), (y1-y0) x n
  *      doubles.  Halo rows travel over NVLink peer memory (CUDA IPC) when every rank can map its neighbours,
- *      over NCCL send/recv otherwise (PMG_P2P=0 forces the latter).  V-, W- and F-cycles, nu <= 2; results are
- *      bit-identical to one GPU (the F-cycle needs equally sized slabs: n_ranks a power of two).
+ *      over NCCL send/recv otherwise (PMG_P2P=0 forces the latter).  V-, W-, F-cycles and the general-RHS FMG pass
+ *      (PMG_CYCLE_FMG, also as the start of pmg_solve), nu <= 2; results are bit-identical to one GPU (the F-cycle and
+ *      the FMG pass need equally sized slabs: n_ranks a power of two).
  *      Failure semantics: a rank that waits longer than PMG_P2P_TIMEOUT_S (environment, default 30 s of device wall time)
  *      for a neighbour's rows gives up, the finest level's iterate of that cycle is NOT committed, and the call -- and
  *      every later call on that handle -- returns PMG_ERR_COMM: the ranks' exchange epochs no longer agree, so the

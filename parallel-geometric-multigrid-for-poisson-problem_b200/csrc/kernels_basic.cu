@@ -11,6 +11,7 @@
 
 #define PMG_NEEDS_PEER_WAIT
 #include "pmg_internal.h"
+#include "kernel_residual_restrict.cuh"
 
 namespace pmg {
 
@@ -1006,6 +1007,16 @@ void launch_restrict(const double *fine, double *coarse, int nf, int nc, int pit
 {
     (void)nf;
     k_restrict<<<grid2d(nc, nc), dim3(BX, BY), 0, st>>>(fine, coarse, nc, nc, 0, pitch_f, pitch_c);
+    count_launch();
+}
+
+void launch_residual_restrict(const double *x, const double *f, double *coarse, int nf, int nc, int rows_c, int yoff_c,
+                              int pitch_x, int pitch_f, int pitch_c, double h, cudaStream_t st)
+{
+    (void)nf;
+    const RRGeom g = residual_restrict_geom(nc, rows_c, yoff_c);
+    if (g.blocks < 1) return;
+    k_residual_restrict<<<g.blocks, RR_WARPS * 32, 0, st>>>(x, f, coarse, nc, g, pitch_x, pitch_f, pitch_c, 1.0 / (h * h));
     count_launch();
 }
 

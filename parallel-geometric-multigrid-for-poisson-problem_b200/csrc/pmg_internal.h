@@ -221,6 +221,11 @@ void launch_restrict_rows(const double *fine, double *coarse, int nc, int rows_c
                           int pitch_c, cudaStream_t st);
 void launch_prolong_add_rows(const double *coarse, double *fine, int nf, int rows_f, int yoff_f, int pitch_c,
                              int pitch_f, int mode, cudaStream_t st);
+// coarse(interior) = R(f - A x) in one pass (kernel_residual_restrict.cuh), bit-identical to launch_residual into a scratch
+// array followed by launch_restrict; 18 B per fine point instead of 34.  Same slab convention as launch_restrict_rows
+// (whole level: rows_c = nc, yoff_c = 0); reads x rows [-2, 2 rows_c] and f rows [-1, 2 rows_c - 1] of the fine window.
+void launch_residual_restrict(const double *x, const double *f, double *coarse, int nf, int nc, int rows_c, int yoff_c,
+                              int pitch_x, int pitch_f, int pitch_c, double h, cudaStream_t st);
 // dst(y,x) = src(y,x) for a ny x nx window, arbitrary pitches (layout conversion at the ABI)
 void launch_copy2d(double *dst, int pitch_d, const double *src, int pitch_s, int nx, int ny,
                    cudaStream_t st);

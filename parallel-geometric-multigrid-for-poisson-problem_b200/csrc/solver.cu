@@ -889,12 +889,10 @@ static pmg_status cycle_f(pmg_solver *s, int *norm_np = nullptr)
 }
 
 // PMG_CYCLE_FMG: one full-multigrid pass for an arbitrary right-hand side and Dirichlet ring (pmg.h; not a
-// reference function -- SURVEY.md 8f-2; specification: the CPU checker's orc_fmg_general).  Scratch: the
-// residual r0 lives in the F-cycle's spare level-0 array; the coarse right-hand sides are the levels' own f arrays.
+// reference function -- SURVEY.md 8f-2; specification: the CPU checker's orc_fmg_general).  The coarse right-hand
+// sides are the levels' own f arrays; r0 = f - A x is never stored (launch_residual_restrict forms R r0 directly).
 static pmg_status cycle_fmg_general(pmg_solver *s)
 {
-    pmg_status rc = ensure_fmg(s);
-    if (rc != PMG_OK) return rc;
     const pmg_config &c = s->cfg;
     const int lc = (int)s->lv.size() - 1;
     Level &L0 = s->lv[0];
@@ -902,16 +900,17 @@ static pmg_status cycle_fmg_general(pmg_solver *s)
     // x = (ring kept, interior 0)
     if (L0.n > 2) launch_fill2d(L0.x + L0.pitch + 1, L0.pitch, L0.n - 2, L0.n - 2, 0.0, s->stream);
     if (lc == 0 || L0.n <= c.n_coarse) return smooth_operator(s, 0, c.coarse_sweeps, false);
-    // r0 = f - A x into the spare array (interior; its ring is never read), then the chain of restrictions
-    s->fmg0_rhs_cached = false;  // the spare level-0 array is scratch here
-    launch_residual(s->f_fmg0, L0.x, L0.f, L0.n, L0.n, L0.pitch, L0.pitch, L0.pitch, L0.h, s->stream);
-    for (int l = 0; l < lc; ++l) {
+    // f_1 = R(f - A x), then the chain of restrictions
+    Level &L1 = s->lv[1];
+    launch_residual_restrict(L0.x, L0.f, L1.f, L0.n, L1.n, L1.n, 0, L0.pitch, L0.pitch, L1.pitch, L0.h, s->stream);
+    for (int l = 1; l < lc; ++l) {
         const Level &L = s->lv[l];
         Level &K = s->lv[l + 1];
-        launch_restrict(l == 0 ? s->f_fmg0 : L.f, K.f, L.n, K.n, L.pitch, K.pitch, s->stream);
+        launch_restrict(L.f, K.f, L.n, K.n, L.pitch, K.pitch, s->stream);
     }
     // coarsest level: coarse_sweeps sweeps from zero
-    if ((rc = smooth_operator(s, lc, c.coarse_sweeps, true)) != PMG_OK) return rc;
+    pmg_status rc = smooth_operator(s, lc, c.coarse_sweeps, true);
+    if (rc != PMG_OK) return rc;
     // upwards: prolongation into a zeroed level, one V-cycle there; on the finest level the true problem (x, f)
     for (int l = lc - 1; l >= 0; --l) {
         Level &K = s->lv[l + 1];
@@ -921,6 +920,76 @@ static pmg_status cycle_fmg_general(pmg_solver *s)
         rc = s->fused ? cycle_fused(s, l, false, false, false, nullptr) : cycle_operator(s, l, false, false);
         if (rc != PMG_OK) return rc;
     }
+    return PMG_OK;
+}
+
+// PMG_CYCLE_FMG on row slabs: the operator sequence of cycle_fmg_general, level by level, under the rules of cycle_f_dist
+// (below): slab levels (l < agg_level) on slabs with an NCCL halo exchange ahead of every slab operator that reads a
+// neighbour row, whole levels redundantly on every rank, the V-cycle of a slab level = cycle_dist started there.  Halo
+// depths: the fused residual-restriction reads 2 x rows and 1 f row beyond the slab, the slab restriction 1 f row, the
+// slab prolongation 1 coarse row below the slab -- which the child's last Pass B (4 finished rows beyond its slab, see
+// cycle_dist) or the whole agglomerated level read in place already holds.  The f halo rows every later cycle_dist(l)
+// reads are the ones exchanged in the chain; nothing rewrites f_l before that cycle.  Every rewrite of an array a
+// neighbour may still read over NVLink (x_l, f_l) has an NCCL collective in between: the exchanges here and the
+// all-gather of the agglomerated level inside each cycle_dist.
+static pmg_status cycle_fmg_dist(pmg_solver *s)
+{
+    if (!s->coarse_redundant)
+        return fail(PMG_ERR_UNSUPPORTED, "multi-GPU FMG pass needs equally sized slabs on the first agglomerated level");
+    const pmg_config &c = s->cfg;
+    const int nl = (int)s->lv.size(), lc = nl - 1, la = s->agg_level;
+    const int *ay0 = s->y0s[la].data(), *ay1 = s->y1s[la].data();
+    Level &A = s->lv[la];
+    Level &L0 = s->lv[0];
+    pmg_status rc;
+    s->cycle_has_collective = false;  // the agglomerated level travels by NCCL all-gather inside these V-cycles
+    drop_graphs(s);                   // the coarsest solve may swap the x / xb roles of a whole level
+    if (s->agg_f[0]) s->aslab.f = s->agg_f[0] + level_origin(s->aslab.n);  // the buffer the NCCL all-gather sends from
+    // (1) x = (ring kept, interior 0) on my rows; halo rows of x and f for the residual
+    {
+        const int ga = std::max(L0.y0, 1), gb = std::min(L0.y0 + L0.ny, L0.n - 1);
+        if (gb > ga) launch_fill2d(L0.x + (ptrdiff_t)(ga - L0.y0) * L0.pitch + 1, L0.pitch, L0.n - 2, gb - ga, 0.0, s->stream);
+        if ((rc = comm_halo_exchange(L0.x, L0.ny, L0.pitch, PADY, s->stream)) != PMG_OK) return rc;
+        if ((rc = comm_halo_exchange(L0.f, L0.ny, L0.pitch, PADY, s->stream)) != PMG_OK) return rc;
+    }
+    // (2) f_1 = R(f - A x) on my coarse rows; (3) f_{l+1} = R f_l down the slab levels, all-gathered into the whole level
+    // the redundant V-cycles read, then restricted redundantly
+    for (int l = 0; l < lc; ++l) {
+        Level &L = s->lv[l];
+        if (l < la) {
+            Level &K = (l + 1 == la) ? s->aslab : s->lv[l + 1];
+            if (l == 0) {
+                launch_residual_restrict(L.x, L.f, K.f, L.n, K.n, K.ny, K.y0, L.pitch, L.pitch, K.pitch, L.h, s->stream);
+            } else {
+                if ((rc = comm_halo_exchange(L.f, L.ny, L.pitch, PADY, s->stream)) != PMG_OK) return rc;
+                launch_restrict_rows(L.f, K.f, K.n, K.ny, K.y0, L.pitch, K.pitch, s->stream);
+            }
+            if (l + 1 == la && (rc = comm_allgather_rows(K.f, A.f, ay1[0] - ay0[0], A.pitch, s->stream)) != PMG_OK) return rc;
+        } else {
+            Level &K = s->lv[l + 1];
+            launch_restrict(L.f, K.f, L.n, K.n, L.pitch, K.pitch, s->stream);
+        }
+    }
+    // (4) coarsest level: coarse_sweeps sweeps from zero, on every rank
+    if ((rc = smooth_operator(s, lc, c.coarse_sweeps, true)) != PMG_OK) return rc;
+    // (5) upwards: e_l = P e_{l+1} into zeros, one V-cycle on (e_l, f_l); (6) level 0: x += P e_1, one V-cycle on (x, f)
+    for (int l = lc - 1; l >= 0; --l) {
+        Level &K = s->lv[l + 1];
+        Level &L = s->lv[l];
+        if (l >= la) {
+            launch_fill2d(L.x, L.pitch, L.n, L.n, 0.0, s->stream);
+            launch_prolong_add(K.x, L.x, K.n, L.n, K.pitch, L.pitch, c.prolong_mode, s->stream);
+            rc = cycle_fused(s, l, false, false, false, nullptr);
+        } else {
+            if (l > 0) PMG_CUDA(cudaMemsetAsync(L.base_x, 0, L.elems * sizeof(double), s->stream));
+            // the coarse iterate: the child slab, or my rows of the whole agglomerated level read in place
+            const double *e = (l + 1 == la) ? A.x + (ptrdiff_t)ay0[s->rank] * A.pitch : K.x;
+            launch_prolong_add_rows(e, L.x, L.n, L.ny, L.y0, K.pitch, L.pitch, c.prolong_mode, s->stream);
+            rc = cycle_dist(s, l, false, false, false, nullptr, nullptr);
+        }
+        if (rc != PMG_OK) return rc;
+    }
+    drop_graphs(s);  // a coarse solve captured above holds x / xb roles the coarsest smoothing may have swapped
     return PMG_OK;
 }
 
@@ -1111,8 +1180,7 @@ static pmg_status run_cycle_inner(pmg_solver *s, pmg_cycle_kind kind, bool want_
 {
     pmg_status rc;
     if (kind == PMG_CYCLE_FMG) {
-        if (s->dist) return fail(PMG_ERR_UNSUPPORTED, "PMG_CYCLE_FMG is single-GPU only");
-        rc = cycle_fmg_general(s);
+        rc = s->dist ? cycle_fmg_dist(s) : cycle_fmg_general(s);
         if (rc == PMG_OK && want_norm) rc = residual_norm2_async(s);
         return rc;
     }
@@ -2437,7 +2505,9 @@ pmg_status pmg_smooth(pmg_solver *s, int sweeps, int block)
 /* Times one fused pass of level `level` in isolation: which = 0 Pass A (sweeps+residual+restriction),
  * 1 Pass B with the residual norm, 2 Pass B without, 3 Pass A with x == 0 (coarse-level form), 4 the cross-cycle pass
  * (Pass B of one cycle + Pass A of the next; level 0, one GPU, x_k not written as in pmg_solve), 5 Pass A with x == 0
- * without the xb store, 6 Pass B rebuilding xb from f (the pair a large first visit runs instead of 3 and 2).  `reps`
+ * without the xb store, 6 Pass B rebuilding xb from f (the pair a large first visit runs instead of 3 and 2), 7 the fused
+ * residual-restriction R(f - A x) of the FMG set-up (one GPU), 8 the residual + restriction pair it replaces (the residual
+ * stored in the level's xb array).  `reps`
  * launches between two CUDA events on the solver stream; *ms_avg = average per launch.  Clobbers the
  * iterate (benchmark use only). */
 pmg_status pmg_bench_pass(pmg_solver *s, int which, int level, int reps, double *ms_avg)
@@ -2455,8 +2525,14 @@ pmg_status pmg_bench_pass(pmg_solver *s, int which, int level, int reps, double 
         pmg_status rcx = ensure_xc(s);
         if (rcx != PMG_OK) return rcx;
     }
+    if ((which == 7 || which == 8) && s->dist) return fail(PMG_ERR_UNSUPPORTED, "forms 7 and 8 time a whole level (one GPU)");
     auto one = [&]() {
-        if (which == 4) {
+        if (which == 7) {
+            launch_residual_restrict(L.x, L.f, K.f, L.n, K.n, K.n, 0, L.pitch, L.pitch, K.pitch, L.h, s->stream);
+        } else if (which == 8) {
+            launch_residual(L.xb, L.x, L.f, L.n, L.n, L.pitch, L.pitch, L.pitch, L.h, s->stream);
+            launch_restrict(L.xb, K.f, L.n, K.n, L.pitch, K.pitch, s->stream);
+        } else if (which == 4) {
             FusedLevel v = fused_view(L);
             v.x = nullptr;
             use_rhs_tables(s, v);  // the flavour pmg_solve runs
@@ -2575,6 +2651,22 @@ pmg_status pmg_test_fused_cross(const pmg_test_slab *t, double *xb_out, const do
     pmg_status rc = require_device();
     if (rc != PMG_OK) return rc;
     launch_fused_cross(test_view(t), xb_out, coarse_x, coarse_f, pitch_c, omega, prolong_mode, d_partials, n_partials, nullptr);
+    PMG_CUDA(cudaDeviceSynchronize());
+    PMG_CUDA(cudaGetLastError());
+    return PMG_OK;
+}
+
+/* the fused residual-restriction of the FMG set-up on caller-built arrays (launch_residual_restrict's arguments): a whole
+ * level (rows_c = nc, yoff_c = 0) or one rank's row-slab window, so that tests/test_gpu_fmg_slabs.py covers the slab path on
+ * one GPU */
+pmg_status pmg_test_residual_restrict(const double *x, const double *f, double *coarse, int nf, int nc, int rows_c, int yoff_c,
+                                      int pitch_x, int pitch_f, int pitch_c, double h)
+{
+    if (!x || !f || !coarse || nf < 3 || nc != (nf - 1) / 2 + 1 || rows_c < 0 || yoff_c < 0 || yoff_c + rows_c > nc)
+        return fail(PMG_ERR_INVALID, "bad argument");
+    pmg_status rc = require_device();
+    if (rc != PMG_OK) return rc;
+    launch_residual_restrict(x, f, coarse, nf, nc, rows_c, yoff_c, pitch_x, pitch_f, pitch_c, h, nullptr);
     PMG_CUDA(cudaDeviceSynchronize());
     PMG_CUDA(cudaGetLastError());
     return PMG_OK;
