@@ -198,7 +198,13 @@ pmg_status pmg_solve(pmg_solver *s, pmg_cycle_kind kind, double rel_tol, int max
  * PMG_PROLONG_FULL, the reference prolongation is not the transpose of the restriction) or not at all (precond = 0: the
  * iteration of ConjugateGradientSmoother, Smoother.hpp:170-256, from the given start).  res_history (nullable,
  * max_iter + 1 doubles): [0] = ||r0||, [k] = ||r_k|| (recurrence residual); stops when ||r_k|| < rel_tol ||r0||.
- * Single GPU.  SURVEY.md 8f-3: "CG as an outer Krylov wrapper preconditioned by one V-cycle". */
+ * On row slabs (n_ranks > 1, any rank count the V-cycle accepts) every rank calls it with the same arguments and works on
+ * its own rows: the iterate it updates and f are this rank's slab, and every rank receives the same history and step
+ * count (the dot products are summed per rank and then in rank order, so every rank stops at the same step).  Against
+ * one GPU, whose sums are grouped differently, the step count is the same in the tested cases, the history agrees to
+ * about 1e-10 relative and the iterate to about 1e-9 of its largest entry -- NOT bit for bit.  A peer-wait time-out
+ * inside the preconditioner is PMG_ERR_COMM, as for the cycles.
+ * SURVEY.md 8f-3: "CG as an outer Krylov wrapper preconditioned by one V-cycle". */
 pmg_status pmg_pcg(pmg_solver *s, int precond, double rel_tol, int max_iter, double *res_history, int *n_iter_out);
 /* device time of the last pmg_solve / pmg_cycle in milliseconds (CUDA events on the solver stream) */
 pmg_status pmg_last_device_ms(pmg_solver *s, double *ms_out);
@@ -249,7 +255,8 @@ int pmg_device_count(void);
  *      doubles.  Halo rows travel over NVLink peer memory (CUDA IPC) when every rank can map its neighbours,
  *      over NCCL send/recv otherwise (PMG_P2P=0 forces the latter).  V-, W-, F-cycles and the general-RHS FMG pass
  *      (PMG_CYCLE_FMG, also as the start of pmg_solve), nu <= 2; results are bit-identical to one GPU (the F-cycle and
- *      the FMG pass need equally sized slabs: n_ranks a power of two).
+ *      the FMG pass need equally sized slabs: n_ranks a power of two).  pmg_pcg runs on slabs too, to a tolerance
+ *      against one GPU (see there).
  *      Failure semantics: a rank that waits longer than PMG_P2P_TIMEOUT_S (environment, default 30 s of device wall time)
  *      for a neighbour's rows gives up, the finest level's iterate of that cycle is NOT committed, and the call -- and
  *      every later call on that handle -- returns PMG_ERR_COMM: the ranks' exchange epochs no longer agree, so the

@@ -333,7 +333,8 @@ class Solver:
 
     def pcg(self, precond=1, rel_tol=1e-8, max_iter=100):
         """Conjugate gradients from the current iterate, preconditioned by one cycle of this solver (precond = 1) or not
-        at all (0); returns (iterations, history)."""
+        at all (0); returns (iterations, history).  On row slabs every rank calls it and updates its own rows
+        (local_rows, get_solution); the history is the global one, the same on every rank."""
         hist = (ctypes.c_double * (max_iter + 1))()
         k = ctypes.c_int()
         L = lib()

@@ -12,6 +12,7 @@
 #define PMG_NEEDS_PEER_WAIT
 #include "pmg_internal.h"
 #include "kernel_residual_restrict.cuh"
+#include "kernel_pcg.cuh"
 
 namespace pmg {
 
@@ -1001,6 +1002,28 @@ void launch_pcg_direction(double *p, const double *z, int nx, int ny, int pitch,
 {
     k_pcg_direction<<<grid2d(nx, ny), dim3(BX, BY), 0, st>>>(p, z, nx, ny, pitch, beta, first ? 1 : 0);
     count_launch();
+}
+
+int launch_pcg_direction_apply(const double *z, const double *p_in, double *p_out, double *ap, int n, int rows, int yoff, int pitch,
+                               double h, const double *beta_num, const double *beta_den, bool first, double *d_partials,
+                               cudaStream_t st)
+{
+    const PDGeom g = pcg_geom(n, rows, yoff);
+    if (g.blocks < 1) return 0;
+    k_pcg_direction_apply<<<g.blocks, PD_WARPS * 32, 0, st>>>(z, p_in, p_out, ap, n, yoff, g, pitch, h * h, beta_num, beta_den,
+                                                             first ? 1 : 0, d_partials);
+    count_launch();
+    return pcg_partials(g);
+}
+
+int launch_pcg_update_dev(double *x, double *r, const double *p, const double *ap, int n, int rows, int yoff, int pitch,
+                          const double *alpha_num, const double *alpha_den, double *d_partials, cudaStream_t st)
+{
+    const PDGeom g = pcg_geom(n, rows, yoff);
+    if (g.blocks < 1) return 0;
+    k_pcg_update_dev<<<g.blocks, PD_WARPS * 32, 0, st>>>(x, r, p, ap, n, g, pitch, alpha_num, alpha_den, d_partials);
+    count_launch();
+    return pcg_partials(g);
 }
 
 void launch_restrict(const double *fine, double *coarse, int nf, int nc, int pitch_f, int pitch_c, cudaStream_t st)

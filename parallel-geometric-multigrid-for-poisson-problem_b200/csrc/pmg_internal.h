@@ -204,6 +204,15 @@ void launch_dot_interior(const double *a, const double *b, int nx, int ny, int p
 void launch_pcg_update(double *x, double *r, const double *p, const double *ap, int nx, int ny, int pitch, double alpha,
                        double *d_partials, double *d_out, cudaStream_t st);
 void launch_pcg_direction(double *p, const double *z, int nx, int ny, int pitch, double beta, bool first, cudaStream_t st);
+// row slabs (kernel_pcg.cuh): the fused direction-operator pass and the update with device-side scalars, on the owned
+// rows [0, rows) of a window whose local row 0 is global row yoff (whole level: rows = n, yoff = 0).  Each writes one
+// partial sum per warp to d_partials (at most PCG_MAX_PARTIALS) and returns their count (0: nothing to do)
+constexpr int PCG_MAX_PARTIALS = 148 * 32;
+int launch_pcg_direction_apply(const double *z, const double *p_in, double *p_out, double *ap, int n, int rows, int yoff, int pitch,
+                               double h, const double *beta_num, const double *beta_den, bool first, double *d_partials,
+                               cudaStream_t st);
+int launch_pcg_update_dev(double *x, double *r, const double *p, const double *ap, int n, int rows, int yoff, int pitch,
+                          const double *alpha_num, const double *alpha_den, double *d_partials, cudaStream_t st);
 
 // *host_ctrl = *ctrl and (host_hist != nullptr) host_hist[0..cycles] = hist2[...], both in mapped pinned host memory,
 // written by a kernel: no copy engine involved (see k_ctrl_to_host)

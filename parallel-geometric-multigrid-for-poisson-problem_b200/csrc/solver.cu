@@ -121,6 +121,9 @@ struct pmg_solver {
     cudaEvent_t ev_staged = nullptr, ev_snap = nullptr, ev_fetched = nullptr, ev_consumed = nullptr;
     bool staged = false, fetching = false;
     double *pcg_base[4] = {nullptr, nullptr, nullptr, nullptr};  // r, z, p, A p of pmg_pcg (level-0 layout; lazily allocated)
+    // pmg_pcg on row slabs (pcg_dist; lazily allocated): the second direction array (the fused direction-operator pass reads
+    // one and writes the other) and [0, 1] r.z of alternate steps, [2] p.Ap, [4 ...] per-warp partial sums
+    double *base_pcg_p2 = nullptr, *d_pcg_sc = nullptr;
     // cross-cycle solve (one GPU, V-cycles): per cycle ONE graph = coarse part from level 1 + the cross-cycle pass on level 0
     // + the convergence kernel; [parity]: which of the two level-0 arrays is the pass's input
     cudaGraphExec_t cross_graph[2] = {nullptr, nullptr};
@@ -1624,6 +1627,8 @@ void pmg_destroy(pmg_solver *s)
     cudaFree(s->base_rhs_sy);
     cudaFree(s->base_f_fmg0);
     for (double *b : s->pcg_base) cudaFree(b);
+    cudaFree(s->base_pcg_p2);
+    cudaFree(s->d_pcg_sc);
     cudaFree(s->base_xc);
     cudaFree(s->base_f_stage);
     cudaFree(s->base_x_snap);
@@ -2249,10 +2254,12 @@ static pmg_status solve_impl(pmg_solver *s, pmg_cycle_kind kind, double rel_tol,
 }
 
 // ---- preconditioned conjugate gradients (pmg.h; specification: the CPU checker's orc_pcg) -----------------------------
+static pmg_status pcg_dist(pmg_solver *s, int precond, double rel_tol, int max_iter, double *res_history, int *n_iter_out);
+
 static pmg_status pcg_impl(pmg_solver *s, int precond, double rel_tol, int max_iter, double *res_history, int *n_iter_out)
 {
     if (!s || max_iter < 0 || (precond != 0 && precond != 1)) return fail(PMG_ERR_INVALID, "bad argument");
-    if (s->dist) return fail(PMG_ERR_UNSUPPORTED, "pmg_pcg is single-GPU only");
+    if (s->dist) return pcg_dist(s, precond, rel_tol, max_iter, res_history, n_iter_out);
     PMG_CUDA(cudaSetDevice(s->device));
     Level &L = s->lv[0];
     for (double *&b : s->pcg_base)
@@ -2320,6 +2327,113 @@ static pmg_status pcg_impl(pmg_solver *s, int precond, double rel_tol, int max_i
     if (n_iter_out) *n_iter_out = k;
     if (precond) drop_graphs(s);  // the operator engine's coarse solves may have swapped x / xb roles below level 0
     return PMG_OK;
+}
+
+// pmg_pcg on row slabs: orc_pcg's step on this rank's owned rows of level 0.  Per step:
+//   precond: exchange PADY halo rows of r, then z = one cycle_dist(0) from zero on (z, r).  With x_is_zero, level 0 does
+//     no halo exchange and its Pass A reads the LOCAL f halo rows, so pointing level 0 at the PCG arrays touches no array
+//     a neighbour maps over NVLink; it also means r's halo must be fresh before every preconditioner cycle;
+//   one row of z beyond the slab from the neighbours (level 0's last Pass B finishes the owned rows only -- cycle_dist:
+//     ext 0 on level 0), which the direction-operator pass reads;
+//   rz = r.z, p = z + beta p with Ap and p.Ap (one fused pass, launch_pcg_direction_apply), x += alpha p and r -= alpha Ap
+//     with r.r.  Every dot product is summed per rank, all-gathered and summed in rank order (launch_final_sum).
+// alpha and beta never leave the GPU: the kernels divide the device-side sums themselves, so a step has ONE device-to-host
+// read, ||r||.  The sums differ from one GPU's only in their grouping, hence the tolerance (not bit identity) in pmg.h.
+static pmg_status pcg_dist(pmg_solver *s, int precond, double rel_tol, int max_iter, double *res_history, int *n_iter_out)
+{
+    PMG_CUDA(cudaSetDevice(s->device));
+    Level &L = s->lv[0];
+    for (double *&b : s->pcg_base)
+        if (!b) {
+            pmg_status rc = alloc_zero(&b, L.elems);
+            if (rc != PMG_OK) return rc;
+        }
+    if (!s->base_pcg_p2) {
+        pmg_status rc = alloc_zero(&s->base_pcg_p2, L.elems);
+        if (rc != PMG_OK) return rc;
+    }
+    if (!s->d_pcg_sc) {
+        pmg_status rc = alloc_zero(&s->d_pcg_sc, 4 + (size_t)PCG_MAX_PARTIALS);
+        if (rc != PMG_OK) return rc;
+    }
+    const size_t o = level_origin(L.n);
+    double *r = s->pcg_base[0] + o, *z_arr = s->pcg_base[1] + o, *ap = s->pcg_base[3] + o;
+    double *pp[2] = {s->pcg_base[2] + o, s->base_pcg_p2 + o};
+    double *sc = s->d_pcg_sc, *part = s->d_pcg_sc + 4;
+    cudaStream_t st = s->stream;
+    // the window whose own "ring" rows are local rows a-1 and b: whole-level interior kernels on the owned interior rows
+    const int ga = std::max(L.y0, 1), gb = std::min(L.y0 + L.ny, L.n - 1), a = ga - L.y0, b = gb - L.y0;
+    const ptrdiff_t wo = (ptrdiff_t)(a - 1) * L.pitch;
+    const int wrows = b - a + 2;
+    // this rank's sum in d_scalar -> the rank-ordered global sum in *dst, the same bits on every rank
+    auto global_sum = [&](double *dst) -> pmg_status {
+        pmg_status rc = comm_allgather_double(s->d_scalar, s->d_gather, st);
+        if (rc == PMG_OK) launch_final_sum(s->d_gather, s->n_ranks, dst, st);
+        return rc;
+    };
+    if (s->p2p)  // Pass B(0) of the preconditioner honours the control block's flag; a finished pmg_solve left it raised
+        PMG_CUDA(cudaMemsetAsync(&s->d_ctrl->done, 0, sizeof(int), st));
+    s->cycle_has_collective = false;  // the agglomerated level travels by NCCL all-gather inside the preconditioner
+    drop_graphs(s);
+    PMG_CUDA(cudaEventRecord(s->ev0, st));
+    pmg_status rc = comm_halo_exchange(L.x, L.ny, L.pitch, PADY, st);
+    if (rc != PMG_OK) return rc;
+    launch_residual(r + wo, L.x + wo, L.f + wo, L.n, wrows, L.pitch, L.pitch, L.pitch, L.h, st);
+    launch_dot_interior(r + wo, r + wo, L.n, wrows, L.pitch, s->d_partials, s->d_scalar, st);
+    if ((rc = global_sum(s->d_scalar)) != PMG_OK) return rc;
+    double rr = 0.0;
+    if ((rc = read_scalar(s, &rr)) != PMG_OK) return rc;
+    const double r0 = std::sqrt(rr);
+    if (res_history) res_history[0] = r0;
+    int k = 0;
+    double rnorm = r0;
+    // every rank reads the same bits of ||r|| (rank-ordered sums), so all take the same branch here and run the same
+    // collectives inside cycle_dist
+    while (k < max_iter && !(rnorm < rel_tol * r0) && r0 > 0.0) {
+        double *z = r;
+        if (precond) {
+            if ((rc = comm_halo_exchange(r, L.ny, L.pitch, PADY, st)) != PMG_OK) return rc;
+            double *sx = L.x, *sbx = L.base_x, *sf = L.f, *sbf = L.base_f;
+            L.x = z_arr;
+            L.base_x = s->pcg_base[1];
+            L.f = r;
+            L.base_f = s->pcg_base[0];
+            rc = cycle_dist(s, 0, false, true, false, nullptr, nullptr);
+            z = L.x;
+            L.x = sx;
+            L.base_x = sbx;
+            L.f = sf;
+            L.base_f = sbf;
+            if (rc != PMG_OK) return rc;
+            if (const int bad = fused_take_bad_nu())
+                return fail(PMG_ERR_UNSUPPORTED, "fused engine: no kernel for " + std::to_string(bad) + " sweeps per pass");
+        }
+        if ((rc = comm_halo_exchange(z, L.ny, L.pitch, 1, st)) != PMG_OK) return rc;
+        double *rz = sc + (k & 1), *rz_prev = sc + ((k & 1) ^ 1), *pap = sc + 2;
+        launch_dot_interior(r + wo, z + wo, L.n, wrows, L.pitch, s->d_partials, s->d_scalar, st);
+        if ((rc = global_sum(rz)) != PMG_OK) return rc;
+        double *p = pp[k & 1];
+        int np = launch_pcg_direction_apply(z, pp[(k & 1) ^ 1], p, ap, L.n, L.ny, L.y0, L.pitch, L.h, rz, rz_prev, k == 0, part,
+                                            st);
+        launch_final_sum(part, np, s->d_scalar, st);
+        if ((rc = global_sum(pap)) != PMG_OK) return rc;
+        np = launch_pcg_update_dev(L.x, r, p, ap, L.n, L.ny, L.y0, L.pitch, rz, pap, part, st);
+        launch_final_sum(part, np, s->d_scalar, st);
+        if ((rc = global_sum(s->d_scalar)) != PMG_OK) return rc;
+        if ((rc = read_scalar(s, &rr)) != PMG_OK) return rc;
+        if ((rc = check_comm_err(s)) != PMG_OK) return rc;  // a timed-out peer wait in the preconditioner
+        ++k;
+        rnorm = std::sqrt(rr);
+        if (res_history) res_history[k] = rnorm;
+    }
+    PMG_CUDA(cudaEventRecord(s->ev1, st));
+    PMG_CUDA(cudaEventSynchronize(s->ev1));
+    float ms = 0.f;
+    PMG_CUDA(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
+    s->last_ms = ms;
+    if (n_iter_out) *n_iter_out = k;
+    drop_graphs(s);  // the coarse solves may have swapped x / xb roles of the whole levels
+    return check_comm_err(s);
 }
 
 pmg_status pmg_pcg(pmg_solver *s, int precond, double rel_tol, int max_iter, double *res_history, int *n_iter_out)
@@ -2667,6 +2781,40 @@ pmg_status pmg_test_residual_restrict(const double *x, const double *f, double *
     pmg_status rc = require_device();
     if (rc != PMG_OK) return rc;
     launch_residual_restrict(x, f, coarse, nf, nc, rows_c, yoff_c, pitch_x, pitch_f, pitch_c, h, nullptr);
+    PMG_CUDA(cudaDeviceSynchronize());
+    PMG_CUDA(cudaGetLastError());
+    return PMG_OK;
+}
+
+/* the fused direction-operator pass of pmg_pcg on row slabs (launch_pcg_direction_apply's arguments) on caller-built arrays:
+ * a whole level (rows = n, yoff = 0) or one rank's window, so that tests/test_gpu_pcg_slabs.py covers the slab path on one
+ * GPU.  beta = *beta_num / *beta_den (device pointers); d_partials: PCG_MAX_PARTIALS doubles; *n_partials = count written */
+pmg_status pmg_test_pcg_direction_apply(const double *z, const double *p_in, double *p_out, double *ap, int n, int rows, int yoff,
+                                        int pitch, double h, const double *beta_num, const double *beta_den, int first,
+                                        double *d_partials, int *n_partials)
+{
+    if (!z || !p_in || !p_out || !ap || !beta_num || !beta_den || !d_partials || !n_partials || n < 3 || rows < 1 ||
+        yoff < 0 || yoff + rows > n)
+        return fail(PMG_ERR_INVALID, "bad argument");
+    pmg_status rc = require_device();
+    if (rc != PMG_OK) return rc;
+    *n_partials = launch_pcg_direction_apply(z, p_in, p_out, ap, n, rows, yoff, pitch, h, beta_num, beta_den, first != 0,
+                                             d_partials, nullptr);
+    PMG_CUDA(cudaDeviceSynchronize());
+    PMG_CUDA(cudaGetLastError());
+    return PMG_OK;
+}
+
+/* the one-GPU pair the fused pass replaces, k_pcg_direction followed by k_apply_a_dot (and its final sum into *d_out), on a
+ * whole level: the baseline tools/pcg_dist_probe.py times the fused pass against */
+pmg_status pmg_test_pcg_direction_pair(const double *z, double *p, double *ap, int n, int pitch, double h, double beta, int first,
+                                       double *d_partials, double *d_out)
+{
+    if (!z || !p || !ap || !d_partials || !d_out || n < 3) return fail(PMG_ERR_INVALID, "bad argument");
+    pmg_status rc = require_device();
+    if (rc != PMG_OK) return rc;
+    launch_pcg_direction(p, z, n, n, pitch, beta, first != 0, nullptr);
+    launch_apply_a_dot(p, ap, n, n, pitch, h, d_partials, d_out, nullptr);
     PMG_CUDA(cudaDeviceSynchronize());
     PMG_CUDA(cudaGetLastError());
     return PMG_OK;
