@@ -198,7 +198,8 @@ pmg_status pmg_solve(pmg_solver *s, pmg_cycle_kind kind, double rel_tol, int max
  * PMG_PROLONG_FULL, the reference prolongation is not the transpose of the restriction) or not at all (precond = 0: the
  * iteration of ConjugateGradientSmoother, Smoother.hpp:170-256, from the given start).  res_history (nullable,
  * max_iter + 1 doubles): [0] = ||r0||, [k] = ||r_k|| (recurrence residual); stops when ||r_k|| < rel_tol ||r0||.
- * On row slabs (n_ranks > 1, any rank count the V-cycle accepts) every rank calls it with the same arguments and works on
+ * On row slabs (n_ranks > 1, any rank count and any sweep counts nu1, nu2 = 1..4 the V-cycle accepts; with 3 or 4 sweeps
+ * the preconditioner uses the deep-sweep slab schedule) every rank calls it with the same arguments and works on
  * its own rows: the iterate it updates and f are this rank's slab, and every rank receives the same history and step
  * count (the dot products are summed per rank and then in rank order, so every rank stops at the same step).  Against
  * one GPU, whose sums are grouped differently, the step count is the same in the tested cases, the history agrees to
@@ -254,7 +255,9 @@ int pmg_device_count(void);
  *      pmg_set_guess / pmg_get_solution then move THIS RANK'S rows [y0, y1) (pmg_partition_rows), (y1-y0) x n
  *      doubles.  Halo rows travel over NVLink peer memory (CUDA IPC) when every rank can map its neighbours,
  *      over NCCL send/recv otherwise (PMG_P2P=0 forces the latter).  V-, W-, F-cycles and the general-RHS FMG pass
- *      (PMG_CYCLE_FMG, also as the start of pmg_solve), nu <= 2; results are bit-identical to one GPU (the F-cycle and
+ *      (PMG_CYCLE_FMG, also as the start of pmg_solve), 1 <= nu1, nu2 <= 4 (3 and 4 sweeps add a halo exchange of the
+ *      coarse iterate on the way up, DESIGN.md section 6a -- checked on CPU models and by its kernels on one GPU, not yet
+ *      run on several GPUs); results are bit-identical to one GPU (the F-cycle and
  *      the FMG pass need equally sized slabs: n_ranks a power of two).  pmg_pcg runs on slabs too, to a tolerance
  *      against one GPU (see there).
  *      Failure semantics: a rank that waits longer than PMG_P2P_TIMEOUT_S (environment, default 30 s of device wall time)

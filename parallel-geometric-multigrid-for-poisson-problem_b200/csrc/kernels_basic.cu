@@ -837,14 +837,21 @@ void launch_cycle_finish(const double *d_partials, int count, SolveCtrl *ctrl, d
     count_launch();
 }
 
-void launch_residual_norm2(const double *x, const double *f, int nx, int ny, int pitch_x, int pitch_f,
-                           double h, double *d_partials, double *d_out, cudaStream_t st)
+int launch_residual_partials(const double *x, const double *f, int nx, int ny, int pitch_x, int pitch_f, double h,
+                             double *d_partials, cudaStream_t st)
 {
     long chunks = (long)((nx + RED_THREADS - 1) / RED_THREADS) * ny;
     int blocks = (int)(chunks < RED_BLOCKS ? chunks : RED_BLOCKS);
     if (blocks < 1) blocks = 1;
     k_residual_norm2<<<blocks, RED_THREADS, 0, st>>>(x, f, nx, ny, pitch_x, pitch_f, 1.0 / (h * h), d_partials);
     count_launch();
+    return blocks;
+}
+
+void launch_residual_norm2(const double *x, const double *f, int nx, int ny, int pitch_x, int pitch_f,
+                           double h, double *d_partials, double *d_out, cudaStream_t st)
+{
+    const int blocks = launch_residual_partials(x, f, nx, ny, pitch_x, pitch_f, h, d_partials, st);
     launch_final_sum(d_partials, blocks, d_out, st);
 }
 

@@ -567,18 +567,44 @@ struct CoarseRow {
     double v[C / 2 + 1];  // coarse columns cc .. cc + C/2
 };
 
-template <int C>
+// CG: through L2 (ld.global.cg) instead of the non-coherent path -- for a coarse array the same pass wrote halo rows into
+template <int C, bool CG = false>
 __device__ __forceinline__ CoarseRow<C> load_coarse(const double *__restrict__ p)
 {
     CoarseRow<C> r;
     if (C == 4) {
-        const double2 t = __ldg(reinterpret_cast<const double2 *>(p));
+        const double2 t = CG ? __ldcg(reinterpret_cast<const double2 *>(p)) : __ldg(reinterpret_cast<const double2 *>(p));
         r.v[0] = t.x;
         r.v[1] = t.y;
     } else {
-        r.v[0] = __ldg(p);
+        r.v[0] = CG ? __ldcg(p) : __ldg(p);
     }
     return r;
+}
+
+// Coarse halo rows of Pass B's up-exchange (deep-sweep slab schedule): the rows at depth rows_from + 1 ..
+// rows_from + rows_count beyond the slab, this lane's coarse columns cc .. cc + C/2 - 1, peer memory -> local halo rows.
+// All loads first (L1-bypassing), then the stores; nyc = coarse rows of the slab.
+template <int C>
+__device__ __forceinline__ void copy_coarse_halo(const HaloPeers &hp, bool up, bool dn, int cc, int nyc, int pitch_c)
+{
+    constexpr int NP = C / 2;
+    const int from = hp.rows_from, cnt = hp.rows_count;
+    double vu[MAX_UP_ROWS][NP], vd[MAX_UP_ROWS][NP];
+#pragma unroll
+    for (int r = 0; r < MAX_UP_ROWS; ++r)
+#pragma unroll
+        for (int p = 0; p < NP; ++p) {
+            if (up && r < cnt) vu[r][p] = __ldcg(hp.x_up + (ptrdiff_t)(-from - 1 - r) * pitch_c + cc + p);
+            if (dn && r < cnt) vd[r][p] = __ldcg(hp.x_dn + (ptrdiff_t)(from + r) * pitch_c + cc + p);
+        }
+#pragma unroll
+    for (int r = 0; r < MAX_UP_ROWS; ++r)
+#pragma unroll
+        for (int p = 0; p < NP; ++p) {
+            if (up && r < cnt) hp.x_keep[(ptrdiff_t)(-from - 1 - r) * pitch_c + cc + p] = vu[r][p];
+            if (dn && r < cnt) hp.x_keep[(ptrdiff_t)(nyc + from + r) * pitch_c + cc + p] = vd[r][p];
+        }
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -814,13 +840,15 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
 // REBUILD = nu1 > 0 (one GPU, first visit, Pass A ran with NO_XB): xb = S^nu1(0; f) is not read but rebuilt from f ahead of
 // the prolongation -- a pointwise sweep (sweep_row_from_zero) and nu1 - 1 sweep stages -- so the pass reads f and e and
 // writes x: 18 B/point, and Pass A drops its 8 B/point xb store.
+// UPX (row slabs, deep-sweep schedule): the coarse iterate's halo rows come from the neighbours in a prologue (hp).
 // ---------------------------------------------------------------------------------------------------
-template <int C, int PF, int MINB, bool SM, int S, bool PROLONG, bool NORM, bool WEIGHTED, int REBUILD = 0>
+template <int C, int PF, int MINB, bool SM, int S, bool PROLONG, bool NORM, bool WEIGHTED, int REBUILD = 0, bool UPX = false>
 __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
     k_up(const double *__restrict__ xb, double *__restrict__ xo, const double *__restrict__ f,
          const double *__restrict__ e, StripGeom g, int pitch_c, int lo, JacobiCoef coef, double inv_h2,
-         double *__restrict__ partials, const int *__restrict__ done)
+         double *__restrict__ partials, const int *__restrict__ done, HaloPeers hp)
 {
+    static_assert(!UPX || (PROLONG && REBUILD == 0), "the up-exchange feeds the prolongation of a slab level");
     constexpr int D1 = REBUILD > 0 ? REBUILD - 1 : 0;  // rebuild sweep stages with a row of delay
     using Feed = typename FeedSelect<C, PF, S + D1, REBUILD == 0, SM>::type;
     pdl_wait();
@@ -862,21 +890,58 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
     bool cprol[C];  // columns that receive a correction
 #pragma unroll
     for (int k = 0; k < C; ++k) cprol[k] = (col + k >= lo) && (col + k <= g.n - 2);
+    const int cc = col >> 1;
+
+    if constexpr (UPX) {
+        // COARSE HALO PROLOGUE (the up-exchange, as Pass A's halo prologue does it for the fine rows).  One thread of the
+        // launch tells the neighbours that MY coarse rows are final -- the child's Pass B ran earlier on this stream --
+        // then only the warps whose prolongation reads coarse rows beyond the slab wait for the neighbours' epoch and
+        // copy the rows the child did not finish into its local halo rows, every load in flight at once.  Each lane
+        // later reads back (through L2) only the coarse columns it wrote itself, so no barrier is needed.
+        if (blockIdx.x == 0 && threadIdx.x == 0 && (hp.pub_up != nullptr || hp.pub_dn != nullptr)) {
+            __threadfence_system();
+            if (hp.pub_up != nullptr) publish_epoch(hp.pub_up, hp.epoch);
+            if (hp.pub_dn != nullptr) publish_epoch(hp.pub_dn, hp.epoch);
+        }
+        // the first copied coarse row above the slab, -(rows_from + 1), enters fine rows -2 (rows_from + 1) and the odd
+        // row after it; the first one below, nyc + rows_from, enters fine row ny + 2 rows_from - 1 (odd: it interpolates
+        // coarse rows nyc + rows_from - 1 and nyc + rows_from) and every row after it
+        const bool need_up = hp.flag_up != nullptr && j_start < -2 * hp.rows_from;
+        const bool need_dn = hp.flag_dn != nullptr && j_end >= g.ny + 2 * hp.rows_from - 1;
+        if (need_up || need_dn) {
+            int ok = 1;
+            if (lane == 0) {
+                if (need_up) ok = wait_flag(hp.flag_up, hp.epoch) ? ok : 0;
+                if (need_dn) ok = wait_flag(hp.flag_dn, hp.epoch) ? ok : 0;
+            }
+            ok = __shfl_sync(0xffffffffu, ok, 0);
+            if (!ok) {
+                if (lane == 0) {
+                    *hp.err = 1;
+                    if (hp.abort != nullptr) *hp.abort = 1;
+                }
+                return;
+            }
+            copy_coarse_halo<C>(hp, need_up, need_dn, cc, g.ny >> 1, pitch_c);
+            // the coarse loads below must not be scheduled ahead of these stores (the same thread reads back the same
+            // addresses, which the hardware keeps in order; the compiler, given __restrict__ on e, need not)
+            asm volatile("" ::: "memory");
+        }
+    }
 
     Feed feed;
     feed.init(xb, f, g.pitch, col, j_start + D1, g.ny + PADY - 1, lane, threadIdx.x >> 5, HaloPeers{}, g.ny);
 
     // coarse rows: ec = row jc, en = row jc+1, eb = prefetch of row jc+2 (raw, before the shuffle)
-    const int cc = col >> 1;
     const int nc_last_row = ((g.ny - 1) >> 1) + PADY;  // last local coarse row in the allocation
     CoarseRow<C> ec, en, eb;
 #pragma unroll
     for (int q = 0; q <= NP; ++q) ec.v[q] = en.v[q] = eb.v[q] = 0.0;
     if (PROLONG) {
         const int jc0 = j_start >> 1;  // j_start even (possibly negative: arithmetic shift == floor)
-        ec = load_coarse<C>(e + (ptrdiff_t)jc0 * pitch_c + cc);
+        ec = load_coarse<C, UPX>(e + (ptrdiff_t)jc0 * pitch_c + cc);
         ec.v[NP] = __shfl_down_sync(0xffffffffu, ec.v[0], 1);
-        eb = load_coarse<C>(e + (ptrdiff_t)(jc0 + 1) * pitch_c + cc);
+        eb = load_coarse<C, UPX>(e + (ptrdiff_t)(jc0 + 1) * pitch_c + cc);
     }
 
     for (int j = j_start; j <= j_end; j += Feed::UNROLL) {
@@ -900,7 +965,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, MINB)
                     en = eb;
                     en.v[NP] = __shfl_down_sync(0xffffffffu, eb.v[0], 1);
                     int nr = min((jj >> 1) + 2, nc_last_row);
-                    eb = load_coarse<C>(e + (ptrdiff_t)nr * pitch_c + cc);
+                    eb = load_coarse<C, UPX>(e + (ptrdiff_t)nr * pitch_c + cc);
 #pragma unroll
                     for (int q = 0; q < NP; ++q) {
                         corr[2 * q] = ec.v[q];
@@ -1398,24 +1463,41 @@ void down_prolong_launch_w(const FusedLevel &lv, const double *e_in, int pitch_e
                HaloPeers{}, e_in, pitch_e, lo);
 }
 
-template <int C, int PF, int MINB, bool SM, int S, bool PROLONG, bool NORM, bool WEIGHTED, int REBUILD = 0>
+template <int C, int PF, int MINB, bool SM, int S, bool PROLONG, bool NORM, bool WEIGHTED, int REBUILD = 0, bool UPX = false>
 void up_launch_k(const FusedLevel &lv, const double *e, int pitch_c, const StripGeom &g, int lo,
                  const JacobiCoef &c, double inv, double *d_partials, const int *done, cudaStream_t st)
 {
-    auto k = k_up<C, PF, MINB, SM, S, PROLONG, NORM, WEIGHTED, REBUILD>;
+    auto k = k_up<C, PF, MINB, SM, S, PROLONG, NORM, WEIGHTED, REBUILD, UPX>;
     int sm = WARPS_PER_CTA * FeedSelect<C, PF, S + (REBUILD > 0 ? REBUILD - 1 : 0), REBUILD == 0, SM>::type::SMEM_PER_WARP;
     PMG_SMEM_ONCE(k, sm);
-    PMG_LAUNCH(k, dim3(grid_for(g)), dim3(32 * WARPS_PER_CTA), sm, st, lv.xb, lv.x, lv.f, e, g, pitch_c, lo, c, inv, d_partials, done);
+    PMG_LAUNCH(k, dim3(grid_for(g)), dim3(32 * WARPS_PER_CTA), sm, st, lv.xb, lv.x, lv.f, e, g, pitch_c, lo, c, inv, d_partials, done,
+               UPX ? lv.hp : HaloPeers{});
 }
 
-template <int C, int PF, int MINB, bool SM, int S, bool PROLONG, bool NORM>
+template <int C, int PF, int MINB, bool SM, int S, bool PROLONG, bool NORM, bool UPX = false>
 void up_launch_one(const FusedLevel &lv, const double *e, int pitch_c, const StripGeom &g, int lo,
                    const JacobiCoef &c, double inv, double *d_partials, const int *done, cudaStream_t st)
 {
     if (c.weighted)
-        up_launch_k<C, PF, MINB, SM, S, PROLONG, NORM, true>(lv, e, pitch_c, g, lo, c, inv, d_partials, done, st);
+        up_launch_k<C, PF, MINB, SM, S, PROLONG, NORM, true, 0, UPX>(lv, e, pitch_c, g, lo, c, inv, d_partials, done, st);
     else
-        up_launch_k<C, PF, MINB, SM, S, PROLONG, NORM, false>(lv, e, pitch_c, g, lo, c, inv, d_partials, done, st);
+        up_launch_k<C, PF, MINB, SM, S, PROLONG, NORM, false, 0, UPX>(lv, e, pitch_c, g, lo, c, inv, d_partials, done, st);
+}
+
+// Pass B with the coarse up-exchange prologue (deep-sweep slab schedule): one shape per sweep count, always prolonging
+template <int C, int PF, int MINB, bool SM, int S>
+void up_upx_launch(const FusedLevel &lv, const double *e, int pitch_c, double omega, int lo, bool norm,
+                   double *d_partials, int *n_partials, const int *done, cudaStream_t st)
+{
+    StripGeom g = make_geom(lv, S + (norm ? 2 : 1), VariantDesc{C, PF, MINB, SM}, lv.ext_lo, lv.ext_hi);
+    JacobiCoef c = jacobi_coef(lv.h, omega);
+    double inv = 1.0 / (lv.h * lv.h);
+    if (norm)
+        up_launch_one<C, PF, MINB, SM, S, true, true, true>(lv, e, pitch_c, g, lo, c, inv, d_partials, done, st);
+    else
+        up_launch_one<C, PF, MINB, SM, S, true, false, true>(lv, e, pitch_c, g, lo, c, inv, d_partials, done, st);
+    count_launch();
+    if (n_partials) *n_partials = norm ? g.n_strips * g.n_chunks : 0;
 }
 
 template <int C, int PF, int MINB, bool SM, int S>
@@ -1738,6 +1820,22 @@ void launch_fused_up(const FusedLevel &lv, const double *coarse_x, int pitch_c, 
             case 2: up_rebuild_dispatch<2, 3, 5, true, 2>(lv, coarse_x, pitch_c, omega, lo, rebuild_nu1, done, st); break;
             case 3: up_rebuild_dispatch<2, 3, 4, true, 3>(lv, coarse_x, pitch_c, omega, lo, rebuild_nu1, done, st); break;
             case 4: up_rebuild_dispatch<2, 2, 4, true, 4>(lv, coarse_x, pitch_c, omega, lo, rebuild_nu1, done, st); break;
+            default: break;
+        }
+        return;
+    }
+    if (lv.hp.x_keep != nullptr) {  // the coarse up-exchange: the Pass B shapes of the other sweep counts and of variant 1
+        if (coarse_x == nullptr || lv.hp.x_keep != coarse_x || lv.hp.rows_count < 1 || lv.hp.rows_count > MAX_UP_ROWS ||
+            lv.hp.rows_from < 0 || lv.ny <= 0) {
+            refuse(0);
+            if (n_partials) *n_partials = 0;
+            return;
+        }
+        switch (nu2) {
+            case 1: up_upx_launch<2, 3, 4, true, 1>(lv, coarse_x, pitch_c, omega, lo, norm, d_partials, n_partials, done, st); break;
+            case 2: up_upx_launch<2, 3, 5, true, 2>(lv, coarse_x, pitch_c, omega, lo, norm, d_partials, n_partials, done, st); break;
+            case 3: up_upx_launch<2, 3, 4, true, 3>(lv, coarse_x, pitch_c, omega, lo, norm, d_partials, n_partials, done, st); break;
+            case 4: up_upx_launch<2, 2, 4, true, 4>(lv, coarse_x, pitch_c, omega, lo, norm, d_partials, n_partials, done, st); break;
             default: break;
         }
         return;

@@ -162,6 +162,9 @@ void launch_residual(double *r, const double *x, const double *f, int nx, int ny
 int reduce_partials();
 void launch_residual_norm2(const double *x, const double *f, int nx, int ny, int pitch_x, int pitch_f,
                            double h, double *d_partials, double *d_out, cudaStream_t st);
+// its first half: the partial sums only; returns how many (<= reduce_partials()) -- reduce with launch_final_sum
+int launch_residual_partials(const double *x, const double *f, int nx, int ny, int pitch_x, int pitch_f, double h,
+                             double *d_partials, cudaStream_t st);
 // same quantity summed in the reference's left-to-right order (bit-identical to the CPU loop; slow)
 void launch_residual_norm2_sequential(const double *x, const double *f, int nx, int ny, int pitch_x, int pitch_f,
                                       double h, double *d_out, cudaStream_t st);
@@ -273,7 +276,12 @@ struct HaloPeers {
                                    // the host writes the visit's epoch to device memory before each graph replay
     int *abort;                    // (nullable) the solve's device-side `done` flag: raised together with *err so that
                                    // the finest level's last pass does not commit an iterate built on stale halo rows
+    // Pass B's up-exchange (deep-sweep slab schedule, x_keep != nullptr in launch_fused_up): x_up / x_dn / x_keep / flags
+    // describe the COARSE iterate, and the prologue copies its rows at depth rows_from + 1 .. rows_from + rows_count
+    // beyond the slab (rows_count <= MAX_UP_ROWS) -- the ones the child's own Pass B did not finish
+    int rows_from, rows_count;
 };
+constexpr int MAX_UP_ROWS = 4;
 
 #if !defined(PMG_HOST_EMULATION) && defined(PMG_NEEDS_PEER_WAIT)
 // Bounded acquire spin on a flag another GPU publishes with st.release.sys.  The bound is WALL time on the device
@@ -319,7 +327,8 @@ struct FusedLevel {
     // [-PADY, ny + PADY); local row 0 is global row yoff.  ext_lo/ext_hi: see StripGeom.
     int ny, yoff, ext_lo, ext_hi;
     int span_lo, span_hi;  // if span_hi > span_lo: write only local rows [span_lo, span_hi) (span_lo even)
-    HaloPeers hp;          // Pass A only: fused halo exchange (wait for the neighbours, read their rows in place)
+    HaloPeers hp;          // Pass A: fused halo exchange (wait for the neighbours, read their rows in place);
+                           // Pass B: the coarse iterate's up-exchange when hp.x_keep != nullptr (see HaloPeers)
     // (nullable; cross-cycle pass, one GPU) f is separable and bit for bit f(y, x) = fx[x] * sy[y] with zeros in the padding:
     // fx addresses logical column 0 of one padded row (pitch doubles), sy logical row 0 of n + 2*PADY entries.  The
     // default shape then forms f in the pass instead of reading it (20 B/point instead of 28).
@@ -344,6 +353,9 @@ void launch_fused_down(const FusedLevel &lv, double *coarse_f, int pitch_c, int 
 // (count returned through *n_partials; reduce with launch_final_sum)
 // rebuild_nu1 > 0 (whole level, coarse_x, no norm): xb is not read but rebuilt as S^nu1(0; f) -- after a Pass A with
 // x_is_zero and store_xb = false
+// lv.hp.x_keep != nullptr (row slabs, deep-sweep schedule): before the prolongation, the coarse prologue publishes
+// lv.hp.epoch, the warps whose rows reach beyond the slab wait for the neighbours' epoch and copy the coarse rows
+// lv.hp.rows_from + 1 .. + rows_count beyond the slab from lv.hp.x_up / x_dn into lv.hp.x_keep (== coarse_x)
 void launch_fused_up(const FusedLevel &lv, const double *coarse_x, int pitch_c, int nu2, double omega,
                      int prolong_mode, double *d_partials, int *n_partials, cudaStream_t st,
                      const int *done = nullptr, int rebuild_nu1 = 0);

@@ -81,7 +81,46 @@ struct Level {
     // (level 0 only) the same for the two arrays the cross-cycle pass alternates between: [0] = xb, [1] = xc
     const double *up_xb[2] = {nullptr, nullptr}, *dn_xb[2] = {nullptr, nullptr};
     int halo_epoch = 0;
+    int up_epoch = 0;  // deep-sweep schedule: up-exchanges of this level's iterate (one per Pass B of the parent)
 };
+
+// ---- slab schedule depths (DESIGN.md section 6) -------------------------------------------------------------------
+// With nu <= 2 the slab cycle recomputes every halo row the way up needs: Pass A finishes xb on 6 rows beyond the slab,
+// Pass B on levels l > 0 finishes x on 4, exactly the coarse rows the parent's prolongation reads.  With 3 or 4 sweeps
+// no such choice exists for an 8-row halo, so the deep-sweep schedule derives the depths from the sweep counts and
+// exchanges the rest of the child's rows on the way up (cycle_dist, k_up's coarse prologue).
+static bool deep_sweeps(const pmg_config &c) { return std::max(c.nu1, c.nu2) >= 3; }
+
+// rows beyond the slab on which Pass A finishes xb: nu1 sweeps eat one of the PADY exchanged rows each (even: the
+// fused passes start their row chunks on even rows)
+static int pass_a_depth(const pmg_config &c) { return deep_sweeps(c) ? (PADY - c.nu1) & ~1 : 6; }
+
+// rows beyond the slab on which Pass B of level l finishes x: the finest level's own rows only; below it as many as
+// the xb depth allows (nu2 sweeps eat one row each; even)
+static int pass_b_ext(const pmg_config &c, int l)
+{
+    if (l == 0) return 0;
+    return deep_sweeps(c) ? std::max(0, (pass_a_depth(c) - c.nu2) & ~1) : 4;
+}
+
+// coarse rows beyond the slab that Pass B of level l reads: it needs xb + P e on ext + nu2 (+1 for the finest level's
+// residual norm) fine rows beyond, and fine row ny + q - 1 (odd) interpolates coarse rows up to depth q / 2 + 1
+static int pass_b_coarse_rows(const pmg_config &c, int l) { return (pass_b_ext(c, l) + c.nu2 + (l == 0 ? 1 : 0)) / 2 + 1; }
+
+// rows of level l + 1's iterate that the deep-sweep schedule exchanges before Pass B of level l (beyond the
+// pass_b_ext(c, l + 1) rows the child finished itself); 0 with nu <= 2.  At most 3 <= MAX_UP_ROWS.
+static int up_exchange_rows(const pmg_config &c, int l)
+{
+    return deep_sweeps(c) ? std::max(0, pass_b_coarse_rows(c, l) - pass_b_ext(c, l + 1)) : 0;
+}
+
+// the finest level's Pass B sums the residual norm itself when xb reaches one row further than its sweeps eat
+static bool pass_b_norm_fits(const pmg_config &c) { return c.nu2 + 1 <= pass_a_depth(c); }
+
+// d_flags inbox (FLAG_SLOTS ints): [2l], [2l+1] = down exchange of level l from the upper / lower neighbour (l < 16),
+// [32 + rank] = gather inbox (n_ranks <= 32), [UP_FLAG_SLOT + 2k], [+1] = up-exchange of level k's iterate (k < 16).
+// The largest grid, N = 32769, has at most 10 slab levels (2 ranks), so every slot is far from its limit.
+constexpr int UP_FLAG_SLOT = 64, FLAG_SLOTS = 96;
 
 }  // namespace pmg
 
@@ -161,7 +200,7 @@ struct pmg_solver {
     bool split_from_env = false;
     bool p2p = false;                        // halo rows are pulled from the neighbours' memory over NVLink
     bool p2p_fused = true;                   // ... by Pass A itself (no pull kernel, no local copy of the x halo)
-    int *d_flags = nullptr;                  // my inbox: [level][from_up, from_dn] epochs published by neighbours
+    int *d_flags = nullptr;                  // my inbox: epochs published by neighbours (layout: UP_FLAG_SLOT)
     int *up_flags = nullptr, *dn_flags = nullptr;  // the neighbours' inboxes (peer mappings)
     int *d_comm_err = nullptr;               // raised by a pull whose wait timed out
     // peer-to-peer all-gather of the first agglomerated level's right-hand side (V-cycles): double-buffered slab
@@ -476,15 +515,20 @@ static void trace_mark(pmg_solver *s, const char *label, int level)
 // which is exactly what the parent's prolongation and this level's second pass read.
 // The exchange runs on `comm_stream` WHILE Pass A works on the interior rows [8, ny-8), which need no halo;
 // the two boundary strips [-6, 8) and [ny-8, ny+6) follow once the halo has landed.
+// Deep-sweep schedule (max(nu1, nu2) >= 3): Pass A finishes pass_a_depth rows, Pass B pass_b_ext rows, and before Pass B
+// of level l the up_exchange_rows(l) coarse rows beyond what the child finished come from the neighbours.
 static pmg_status cycle_dist(pmg_solver *s, int l, bool w_form, bool x_is_zero, bool want_norm, int *n_partials,
                              const int *done);
+static pmg_status up_exchange(pmg_solver *s, int k, int m, FusedLevel &v);
 
 // First level of the middle graph: the smallest lg >= 1 such that the slab levels lg .. agg_level-1 all run on the
 // compute stream alone (no interior / boundary split, hence no cross-stream events); 0 = no graph.
 static int mid_graph_first_level(const pmg_solver *s, bool w_form)
 {
+    // (not with the deep-sweep schedule: d_epochs holds one halo epoch per level, and its up-exchange would need a
+    // second one; the graph only trims launch latency on short slab levels, measured for nu = 2)
     if (!s->mid_graph_on || w_form || !s->p2p || !s->p2p_fused || !s->p2p_gather || !s->coarse_redundant ||
-        !s->cycle_has_collective || s->d_epochs == nullptr || g_trace_on == 1 || !s->cfg.use_graph)
+        !s->cycle_has_collective || s->d_epochs == nullptr || g_trace_on == 1 || !s->cfg.use_graph || deep_sweeps(s->cfg))
         return 0;
     int lg = s->agg_level;
     while (lg > 1 && s->lv[lg - 1].ny < s->split_min_rows) --lg;
@@ -547,6 +591,7 @@ static pmg_status cycle_dist(pmg_solver *s, int l, bool w_form, bool x_is_zero, 
     const bool last_slab = (l + 1 == s->agg_level);
     Level &K = last_slab ? s->aslab : s->lv[l + 1];
     const bool up_nb = s->rank > 0, dn_nb = s->rank < s->n_ranks - 1;
+    const int da = pass_a_depth(c);
     pmg_status rc;
     trace_mark(s, "begin", l);
     // NVLink all-gather of the agglomerated level into the double-buffered slab.  Two buffers are enough for ANY
@@ -623,14 +668,14 @@ static pmg_status cycle_dist(pmg_solver *s, int l, bool w_form, bool x_is_zero, 
         if (split) {
             v.hp = hp;
             if (up_nb) {
-                v.span_lo = -6;
+                v.span_lo = -da;
                 v.span_hi = PADY;
                 launch_fused_down(v, K.f, K.pitch, c.nu1, c.omega, x_is_zero, s->comm_stream, nullptr);
                 v.hp.pub_up = v.hp.pub_dn = nullptr;  // published once
             }
             if (dn_nb) {
                 v.span_lo = L.ny - PADY;
-                v.span_hi = L.ny + 6;
+                v.span_hi = L.ny + da;
                 launch_fused_down(v, K.f, K.pitch, c.nu1, c.omega, x_is_zero, s->comm_stream, nullptr);
             }
             v.hp = HaloPeers{};
@@ -648,8 +693,8 @@ static pmg_status cycle_dist(pmg_solver *s, int l, bool w_form, bool x_is_zero, 
     } else if (!skip_pass_a) {
         if (halo_on_comm) PMG_CUDA(cudaStreamWaitEvent(s->stream, s->ev_halo, 0));
         trace_mark(s, "halo", l);
-        v.span_lo = up_nb ? -6 : 0;
-        v.span_hi = dn_nb ? L.ny + 6 : L.ny;
+        v.span_lo = up_nb ? -da : 0;
+        v.span_hi = dn_nb ? L.ny + da : L.ny;
         v.hp = halo_peers;  // fused exchange (null when the halo rows were copied in)
         launch_fused_down(v, K.f, K.pitch, c.nu1, c.omega, x_is_zero, s->stream, nullptr);
         trace_mark(s, "passA", l);
@@ -698,7 +743,7 @@ static pmg_status cycle_dist(pmg_solver *s, int l, bool w_form, bool x_is_zero, 
     }
     {
         FusedLevel v = fused_view(L);
-        const int e = (l == 0) ? 0 : 4;
+        const int e = pass_b_ext(c, l);
         v.ext_lo = up_nb ? e : 0;
         v.ext_hi = dn_nb ? e : 0;
         // coarse correction: the child slab's iterate, or -- below the last slab level, where every rank holds the
@@ -738,11 +783,64 @@ static pmg_status cycle_dist(pmg_solver *s, int l, bool w_form, bool x_is_zero, 
                                guard);
             ++s->cross_count;
         } else {
-            launch_fused_up(v, coarse_x, K.pitch, c.nu2, c.omega, c.prolong_mode, want_norm ? s->d_partials : nullptr,
+            // deep-sweep schedule: the child slab's rows beyond those its Pass B finished (the whole agglomerated level
+            // is read in place and needs none)
+            const int m = last_slab ? 0 : up_exchange_rows(c, l);
+            if (m > 0 && (rc = up_exchange(s, l + 1, m, v)) != PMG_OK) return rc;
+            const bool fused_norm = want_norm && pass_b_norm_fits(c);
+            launch_fused_up(v, coarse_x, K.pitch, c.nu2, c.omega, c.prolong_mode, fused_norm ? s->d_partials : nullptr,
                             n_partials, s->stream, l == 0 ? guard : nullptr);
+            if (want_norm && !fused_norm) {
+                // xb does not reach the extra row the fused norm reads (nu1 + nu2 = 7, 8): sum (f - A x)^2 over the owned
+                // rows in a pass of its own, after an exchange of one row of the new iterate
+                if ((rc = comm_halo_exchange(L.x, L.ny, L.pitch, 1, s->stream)) != PMG_OK) return rc;
+                const int ga = std::max(L.y0, 1), gb = std::min(L.y0 + L.ny, L.n - 1);  // owned interior rows
+                const int a = ga - L.y0, b = gb - L.y0;
+                const int np = launch_residual_partials(L.x + (ptrdiff_t)(a - 1) * L.pitch, L.f + (ptrdiff_t)(a - 1) * L.pitch,
+                                                        L.n, b - a + 2, L.pitch, L.pitch, L.h, s->d_partials, s->stream);
+                if (n_partials) *n_partials = np;
+            }
         }
     }
     trace_mark(s, "passB", l);
+    return PMG_OK;
+}
+
+// Deep-sweep schedule: rows pass_b_ext(k) + 1 .. + m beyond the slab of level k's iterate from the neighbours, before
+// Pass B of level k - 1 (v: that pass) reads them.  Over NVLink with PMG_P2P_FUSED on (default) in Pass B's coarse
+// prologue; with a pull kernel ahead of it otherwise; by NCCL without peer access.  The last two move all
+// pass_b_ext(k) + m rows, each side one contiguous block.  Every rank runs the same sequence of cycles, so the epochs
+// agree; a neighbour re-writes its rows only after its next Pass A of level k waited for this rank's epoch of that
+// level, which this rank publishes after the pass below.
+static pmg_status up_exchange(pmg_solver *s, int k, int m, FusedLevel &v)
+{
+    Level &K = s->lv[k];
+    const bool up_nb = s->rank > 0, dn_nb = s->rank < s->n_ranks - 1;
+    const int from = pass_b_ext(s->cfg, k);
+    if (!s->p2p) return comm_halo_exchange(K.x, K.ny, K.pitch, from + m, s->stream);
+    const int epoch = ++K.up_epoch;
+    const int slot = UP_FLAG_SLOT + 2 * k;
+    if (!s->p2p_fused) {
+        launch_halo_signal(up_nb ? s->up_flags + slot + 1 : nullptr, dn_nb ? s->dn_flags + slot : nullptr, epoch, s->stream);
+        launch_halo_pull(K.x, K.ny, K.pitch, from + m, up_nb ? K.up_x + (ptrdiff_t)(PADY - from - m) * K.pitch : nullptr,
+                         dn_nb ? K.dn_x : nullptr, s->d_flags + slot, s->d_flags + slot + 1, epoch, s->d_comm_err, s->stream,
+                         &s->d_ctrl->done);
+        return PMG_OK;
+    }
+    HaloPeers hp{};
+    hp.x_up = up_nb ? K.up_x + (ptrdiff_t)PADY * K.pitch : nullptr;
+    hp.x_dn = dn_nb ? K.dn_x : nullptr;
+    hp.x_keep = K.x;
+    hp.flag_up = up_nb ? s->d_flags + slot : nullptr;
+    hp.flag_dn = dn_nb ? s->d_flags + slot + 1 : nullptr;
+    hp.pub_up = up_nb ? s->up_flags + slot + 1 : nullptr;
+    hp.pub_dn = dn_nb ? s->dn_flags + slot : nullptr;
+    hp.epoch = epoch;
+    hp.err = s->d_comm_err;
+    hp.abort = &s->d_ctrl->done;  // a timed-out wait also stops the finest level's Pass B from committing
+    hp.rows_from = from;
+    hp.rows_count = m;
+    v.hp = hp;
     return PMG_OK;
 }
 
@@ -931,7 +1029,8 @@ static pmg_status cycle_fmg_general(pmg_solver *s)
 // neighbour row, whole levels redundantly on every rank, the V-cycle of a slab level = cycle_dist started there.  Halo
 // depths: the fused residual-restriction reads 2 x rows and 1 f row beyond the slab, the slab restriction 1 f row, the
 // slab prolongation 1 coarse row below the slab -- which the child's last Pass B (4 finished rows beyond its slab, see
-// cycle_dist) or the whole agglomerated level read in place already holds.  The f halo rows every later cycle_dist(l)
+// cycle_dist; with the deep-sweep schedule an exchange of the child's halo) or the whole agglomerated level read in
+// place already holds.  The f halo rows every later cycle_dist(l)
 // reads are the ones exchanged in the chain; nothing rewrites f_l before that cycle.  Every rewrite of an array a
 // neighbour may still read over NVLink (x_l, f_l) has an NCCL collective in between: the exchanges here and the
 // all-gather of the agglomerated level inside each cycle_dist.
@@ -985,7 +1084,10 @@ static pmg_status cycle_fmg_dist(pmg_solver *s)
             rc = cycle_fused(s, l, false, false, false, nullptr);
         } else {
             if (l > 0) PMG_CUDA(cudaMemsetAsync(L.base_x, 0, L.elems * sizeof(double), s->stream));
-            // the coarse iterate: the child slab, or my rows of the whole agglomerated level read in place
+            // the coarse iterate: the child slab, or my rows of the whole agglomerated level read in place.  The
+            // deep-sweep schedule's Pass B may finish no row beyond the child slab: its halo rows are exchanged.
+            if (l + 1 < la && deep_sweeps(c) && (rc = comm_halo_exchange(K.x, K.ny, K.pitch, PADY, s->stream)) != PMG_OK)
+                return rc;
             const double *e = (l + 1 == la) ? A.x + (ptrdiff_t)ay0[s->rank] * A.pitch : K.x;
             launch_prolong_add_rows(e, L.x, L.n, L.ny, L.y0, K.pitch, L.pitch, c.prolong_mode, s->stream);
             rc = cycle_dist(s, l, false, false, false, nullptr, nullptr);
@@ -1301,10 +1403,10 @@ pmg_status pmg_create(const pmg_config *cfg, pmg_solver **out)
     if (dist) {
         if (!comm_ready() || comm_size() != cfg->n_ranks || comm_rank() != cfg->rank)
             return fail(PMG_ERR_INVALID, "n_ranks > 1 needs pmg_comm_init with the same rank / n_ranks first");
-        if (cfg->engine != PMG_ENGINE_FUSED || !(cfg->nu1 >= 1 && cfg->nu1 <= 2 && cfg->nu2 >= 1 && cfg->nu2 <= 2) ||
+        if (cfg->engine != PMG_ENGINE_FUSED || !(cfg->nu1 >= 1 && cfg->nu1 <= 4 && cfg->nu2 >= 1 && cfg->nu2 <= 4) ||
             cfg->smoother_eps > 0.0 || cfg->norm_mode != PMG_NORM_TREE)
             return fail(PMG_ERR_UNSUPPORTED,
-                        "multi-GPU: fused engine, 1-2 pre/post sweeps, smoother_eps = 0 and the tree norm only");
+                        "multi-GPU: fused engine, 1-4 pre/post sweeps, smoother_eps = 0 and the tree norm only");
     }
     int ndev = pmg_device_count();
     if (ndev <= 0) return fail(PMG_ERR_NO_DEVICE, "no CUDA device visible; this library has no CPU fallback");
@@ -1467,8 +1569,8 @@ pmg_status pmg_create(const pmg_config *cfg, pmg_solver **out)
             // is exported with CUDA IPC: the inbox flags, the x / f slab arrays of every partitioned level and the
             // two buffers of the first agglomerated level's right-hand side.
             const int R = cfg->n_ranks, me = cfg->rank;
-            bool ok = cudaMalloc((void **)&s->d_flags, 64 * sizeof(int)) == cudaSuccess &&
-                      cudaMemset(s->d_flags, 0, 64 * sizeof(int)) == cudaSuccess &&
+            bool ok = cudaMalloc((void **)&s->d_flags, FLAG_SLOTS * sizeof(int)) == cudaSuccess &&
+                      cudaMemset(s->d_flags, 0, FLAG_SLOTS * sizeof(int)) == cudaSuccess &&
                       cudaMalloc((void **)&s->d_epochs, 16 * sizeof(int)) == cudaSuccess &&
                       cudaMemset(s->d_epochs, 0, 16 * sizeof(int)) == cudaSuccess &&
                       // mapped pinned HOST memory: kernels store to it only when a peer wait times out, the host
@@ -2751,6 +2853,32 @@ pmg_status pmg_test_fused_up(const pmg_test_slab *t, const double *coarse_x, int
     FusedLevel v = test_view(t);
     v.hp = HaloPeers{};
     launch_fused_up(v, coarse_x, pitch_c, nu2, omega, prolong_mode, d_partials, n_partials, nullptr);
+    PMG_CUDA(cudaDeviceSynchronize());
+    PMG_CUDA(cudaGetLastError());
+    return PMG_OK;
+}
+
+/* Pass B with the deep-sweep schedule's coarse up-exchange on a caller-built slab: t->x / xb / f / ext as for
+ * pmg_test_fused_up; t->x_up / x_dn / flags / pubs / epoch / err describe the COARSE iterate coarse_x (its neighbours'
+ * copies, as cycle_dist passes them: x_up = the upper neighbour's coarse row ny_up), whose rows rows_from + 1 ..
+ * rows_from + rows_count beyond the slab the prologue copies in.  abort (nullable): raised with err on a time-out. */
+pmg_status pmg_test_fused_up_exchange(const pmg_test_slab *t, double *coarse_x, int pitch_c, int nu2, double omega,
+                                      int prolong_mode, double *d_partials, int *n_partials, int rows_from, int rows_count,
+                                      int *abort)
+{
+    if (!t || !coarse_x || !fused_supported(nu2) || rows_from < 0 || rows_count < 1 || rows_count > MAX_UP_ROWS || t->ny <= 0)
+        return fail(PMG_ERR_INVALID, "bad argument");
+    pmg_status rc = require_device();
+    if (rc != PMG_OK) return rc;
+    FusedLevel v = test_view(t);
+    v.hp.f_up = v.hp.f_dn = nullptr;
+    v.hp.f_keep = nullptr;
+    v.hp.x_keep = coarse_x;
+    v.hp.abort = abort;
+    v.hp.rows_from = rows_from;
+    v.hp.rows_count = rows_count;
+    launch_fused_up(v, coarse_x, pitch_c, nu2, omega, prolong_mode, d_partials, n_partials, nullptr);
+    if (fused_take_bad_nu()) return fail(PMG_ERR_UNSUPPORTED, "Pass B with the up-exchange refused these arguments");
     PMG_CUDA(cudaDeviceSynchronize());
     PMG_CUDA(cudaGetLastError());
     return PMG_OK;
